@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Pix2Pix GAN training throughput (images/sec at 256^2) on N B200s of one box.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): Pix2Pix U-Net (54.4 M params) + PatchGAN (2.76 M), one full GAN
 training step of the reference's ``UnetWrapper.training_step`` (models/wrapper.py:117-162: frozen-G forward,
@@ -13,6 +13,10 @@ with inputs resident in HBM, ``e2e`` = the same through the public API with pinn
 step's batch, prefetched on a copy stream) and a D2H read of every step's loss (issued on a side stream behind the
 step, consumed one iteration later so the host never stalls the GPU), ``roofline`` = the tcgen05 implicit-GEMM kernels' algorithmic TFLOP/s against the
 measured bf16 peak, ``cpu_baseline`` = the oracle's CPU restatement of the reference step on the host cores.
+
+``--dump-outputs DIR`` writes what the last timed step computed as ``DIR/<name>.npy`` (see ``dump_outputs``).  That
+step starts from the seeded initial weights and a fresh optimizer state, and its batch is seeded, so its inputs are the
+same in every run: two runs, or two builds, with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -27,6 +31,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(ROOT, "thesis-pai-reconstruction_b200"))
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 import torch.nn.functional as F  # noqa: E402
 
@@ -112,6 +117,34 @@ class ClockSampler:
         return {"sm_mhz": med, "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons), "samples": len(self.samples)}
 
 
+def dump_outputs(out_dir, logged):
+    """Writes what one training step hands its caller, the values it logged, as ``<name>.npy`` (float32).  The trained
+    weights are not written: Adam's normalised update turns a gradient that is zero up to rounding (the shift of a
+    BatchNorm whose output feeds another BatchNorm) into a full step of either sign, so they differ from run to run
+    by +-lr even from identical inputs."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, values in logged.items():
+        np.save(os.path.join(out_dir, name + ".npy"), torch.as_tensor(values[-1]).detach().float().cpu().numpy())
+
+
+def reset_training_state(model, initial):
+    """Puts ``model`` back to the weights and buffers of ``initial`` (a state_dict) with a fresh optimizer state, all in
+    place, so that a captured step graph keeps working: its next step computes what a first training step does."""
+    from pai_b200 import engine
+    with torch.no_grad():
+        for k, v in model.state_dict().items():
+            v.copy_(initial[k])
+        for p in model.parameters():
+            engine.repack_in_place(p)
+        opts = model.optimizers()
+        for opt in (opts if isinstance(opts, list) else [opts]):
+            for st in opt.state.values():
+                for t in st.values():
+                    t.zero_()                           # step, exp_avg, exp_avg_sq
+            for ent in opt.__dict__.get("_pai_dev", {}).values():
+                ent["step"].zero_()                     # the device-side step counter of FusedAdam
+
+
 def physical_index(local_rank):
     vis = os.environ.get("CUDA_VISIBLE_DEVICES")
     if vis:
@@ -123,9 +156,10 @@ def physical_index(local_rank):
 
 
 # ------------------------------------------------------------------------------------------ CPU arms
-def cpu_reference_step_rate(steps, warmup, batch):
+def cpu_reference_step_rate(steps, warmup, batch, dump=None):
     """The reference's training step on the host cores, via the oracle's CPU restatement
-    (oracle/pix2pix_port.py, pinned to the unmodified reference by tests/golden).  Returns images/s."""
+    (oracle/pix2pix_port.py, pinned to the unmodified reference by tests/golden).  Returns images/s.
+    With ``dump`` a directory, the last step's outputs are written there (``dump_outputs``)."""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import pix2pix_port as port
     cores = os.cpu_count() or 1
@@ -140,6 +174,8 @@ def cpu_reference_step_rate(steps, warmup, batch):
         t0 = time.perf_counter()
         tr.training_step(x, target)
         times.append(time.perf_counter() - t0)
+    if dump:
+        dump_outputs(dump, tr.logged)
     total = sum(times)
     return batch * steps / total, total / steps, cores, torch.get_num_threads()
 
@@ -149,9 +185,9 @@ def run_reference_arm(args):
     if rank != 0:
         return
     batch = args.batch   # the SAME per-GPU batch as our arm (64): about 3-4 s per step on the box's host cores
-    steps = max(1, min(args.steps, 20))
+    steps = args.steps
     warmup = max(1, min(args.warmup, 2))
-    rate, sec, cores, threads = cpu_reference_step_rate(steps, warmup, batch)
+    rate, sec, cores, threads = cpu_reference_step_rate(steps, warmup, batch, dump=args.dump_outputs)
     line = {
         "impl": "reference", "metric": METRIC, "value": rate, "unit": "images/s", "n_gpus": args.gpus,
         "steps": steps, "warmup": warmup, "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -388,6 +424,7 @@ def run_ours(args):
     model = build_model().to(dev)
     dp.broadcast_parameters(model)
     model.train()
+    initial = {k: v.detach().clone() for k, v in model.state_dict().items()} if args.dump_outputs else None
 
     nbatches = 4
     host = [synthetic_pairs(B, seed=1234 + 100 * rank + i) for i in range(nbatches)]
@@ -482,17 +519,30 @@ def run_ours(args):
     torch.cuda.synchronize()
     sampler.start()
     launches0 = lib.launches
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    for i in range(args.steps):
+    # With --dump-outputs the last timed step starts from the seeded initial weights and a fresh optimizer state, put
+    # back between two timed windows: the steps before it sum their gradient atomics in a different order in every
+    # run, so only a reset gives that step the same inputs in every run.
+    split = args.steps - 1 if args.dump_outputs else args.steps
+    ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
+    ev[0].record()
+    for i in range(split):
         step_resident(i)
         model.logged.clear()
-    e1.record()
+    ev[1].record()
+    if split < args.steps:
+        reset_training_state(model, initial)
+        ev[2].record()
+        step_resident(split)
+        ev[3].record()
     torch.cuda.synchronize()
     dp.barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model.logged)
+    model.logged.clear()
     launches = lib.launches - launches0
-    ms_total = dp.allreduce_max(e0.elapsed_time(e1), dev)
+    ms_window = ev[0].elapsed_time(ev[1]) + (ev[2].elapsed_time(ev[3]) if split < args.steps else 0.0)
+    ms_total = dp.allreduce_max(ms_window, dev)
     ms_step = ms_total / args.steps
     value = world * B * args.steps / (ms_total * 1e-3)
 
@@ -619,7 +669,12 @@ def main():
     ap.add_argument("--no-variants", action="store_true", help="skip the Res / Attention / Trans U-Net step rates")
     ap.add_argument("--no-gpu-reference", action="store_true", help="skip the PyTorch eager + cuDNN competitor on this GPU")
     ap.add_argument("--no-graph", action="store_true", help="time eager kernel launches instead of the CUDA-graph step")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="run the last timed step from the initial weights and write the values it logged "
+                         "as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -10,29 +10,35 @@ for p in (ROOT, PKG, os.path.join(ROOT, "oracle")):
         sys.path.insert(0, p)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE = "/root/reference"
+# a checkout of the original thesis-pai-reconstruction project, for the tests that import its modules directly
+REFERENCE = os.environ.get("PAI_REFERENCE_DIR", "")
 
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
+    config.addinivalue_line("markers", "reference: needs a checkout of the original project in $PAI_REFERENCE_DIR")
 
 
 def pytest_collection_modifyitems(config, items):
     import torch
 
     has_gpu = torch.cuda.is_available()
-    has_ref = os.path.isdir(REFERENCE)
+    has_ref = bool(REFERENCE) and os.path.isdir(REFERENCE)
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
         if "reference" in item.keywords and not has_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present on this box"))
+            item.add_marker(pytest.mark.skip(reason="PAI_REFERENCE_DIR does not name a checkout of the original project"))
 
 
 @pytest.fixture(scope="session")
 def golden_dir():
     return GOLDEN
+
+
+@pytest.fixture(scope="session")
+def reference_dir():
+    return REFERENCE
 
 
 @pytest.fixture(scope="session")

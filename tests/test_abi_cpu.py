@@ -52,11 +52,10 @@ def test_version_and_error_channel_without_gpu(so):
     assert rc != 0 and b"11x11 window" in so.pai_last_error()
 
 
-def test_no_cpu_fallback_in_product_metrics():
+def test_no_cpu_fallback_in_product_metrics(monkeypatch):
     import torch
     from pai_b200 import metrics
-    if torch.cuda.is_available():
-        pytest.skip("CUDA present")
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)     # a machine without a CUDA device
     with pytest.raises(RuntimeError, match="no CPU fallback"):
         metrics.ssim(torch.rand(1, 1, 32, 32), torch.rand(1, 1, 32, 32))
 

@@ -9,10 +9,12 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_reference_arm_prints_one_json_line_with_the_contract_keys():
-    """`bench.py --impl reference` times the reference's CPU path (oracle port) and prints exactly one JSON line."""
+def test_reference_arm_prints_one_json_line_with_the_contract_keys(tmp_path):
+    """`bench.py --impl reference` times the reference's CPU path (oracle port) and prints exactly one JSON line;
+    --dump-outputs writes the values the last step logged."""
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",
-                          "--warmup", "1", "--batch", "8"], capture_output=True, text=True, timeout=600, cwd=ROOT)
+                          "--warmup", "1", "--batch", "8", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [ln for ln in out.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1, out.stdout
@@ -23,6 +25,17 @@ def test_reference_arm_prints_one_json_line_with_the_contract_keys():
     assert d["e2e"] == {"value": d["value"], "unit": "images/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert "workload" in d["config"] and d["n_gpus"] == 1 and d["steps"] == 1 and d["warmup"] == 1
     assert d["config"]["batch_per_gpu"] == 8      # the arm runs the batch it is given (default: 64, the same as our arm)
+    check_dumped_outputs(tmp_path)
+
+
+def check_dumped_outputs(out_dir):
+    """What `bench.py --dump-outputs` writes for the GAN step: the five values it logged, float32 scalars."""
+    import numpy as np
+    arrays = {p.name[:-4]: np.load(p) for p in out_dir.iterdir()}
+    assert set(arrays) == {"d_loss", "loss", "train_ssim", "train_psnr", "train_rmse"}
+    for name, a in arrays.items():
+        assert a.dtype == np.float32 and a.shape == () and np.isfinite(a), name
+    assert 0 < arrays["train_ssim"] < 1 and arrays["train_rmse"] > 0
 
 
 def test_reference_arm_other_ranks_exit_quietly():

@@ -1,6 +1,6 @@
 """Pins oracle/pix2pix_port.py (the travelling CPU restatement of the reference's Pix2Pix
 training path) against fixtures produced by the real reference (oracle/gen_golden.py) and,
-when /root/reference is mounted, against the reference modules directly."""
+when $PAI_REFERENCE_DIR names a checkout of it, against the reference modules directly."""
 import os
 import sys
 
@@ -74,11 +74,11 @@ def test_three_training_steps(gz, loss_type, prefix):
 
 
 @pytest.mark.reference
-def test_against_live_reference(state):
+def test_against_live_reference(state, reference_dir):
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     import torchvision  # noqa: F401  (its import inspects sys.modules; do it before the namespace swap)
     sys.path.insert(0, os.path.join(root, "oracle", "shim"))
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, reference_dir)
     saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "models" or k.startswith("models.")}
     # the reference's ``models`` is a namespace package (no __init__.py): a regular package of the same
     # name anywhere on sys.path would win, so the drop-in package's directory steps aside for this test
@@ -108,5 +108,5 @@ def test_against_live_reference(state):
             del sys.modules[k]
         sys.modules.update(saved)
         sys.path[:0] = hidden
-        sys.path.remove("/root/reference")
+        sys.path.remove(reference_dir)
         sys.path.remove(os.path.join(root, "oracle", "shim"))

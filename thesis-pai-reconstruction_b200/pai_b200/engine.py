@@ -94,6 +94,20 @@ def restamp_packs(p: torch.Tensor) -> None:
         store[tag] = (stamp, store[tag][1])
 
 
+def repack_in_place(p: torch.Tensor) -> None:
+    """Rewrites the packs that FusedAdam refreshes in place (see ``fused_pack_targets``) from the current values of
+    ``p``, into the same buffers: for a parameter overwritten in place while a captured step graph keeps reading them.
+    The other packs need nothing: the graph rebuilds them from the parameter at every replay."""
+    if fused_pack_targets(p) is None:
+        return
+    fns = {"conv_f": ops.pack_conv_weight, "convT_d": ops.pack_conv_weight,
+           "conv_d": ops.pack_convT_weight, "convT_f": ops.pack_convT_weight}
+    with torch.no_grad():
+        for tag, (_, buf) in p.__dict__["_pai_packs"].items():
+            buf.copy_(fns[tag](p.detach()))
+    restamp_packs(p)
+
+
 def _fprop_pack(w):      # Conv2d weight [Cout, Cin, 4, 4]
     return _packs.get("conv_f", w, ops.pack_conv_weight)
 

@@ -18,6 +18,8 @@ drops the graph and re-captures when any of them changed (``load_state_dict``, `
 """
 from __future__ import annotations
 
+import gc
+
 import torch
 
 from . import lib
@@ -79,6 +81,12 @@ class StepGraph:
         self._drop_lazy_packs()
         ent.signature = self._signature()
         torch.cuda.synchronize()
+        # A discarded module with its StepGraph is a reference cycle that only the cyclic garbage collector frees, CUDA
+        # graphs included; destroying a graph while this one is being captured invalidates the capture.  So dead cycles
+        # are collected now and the collector stays off until the capture ends.
+        gc.collect()
+        gc_enabled = gc.isenabled()
+        gc.disable()
         sink = []
         m.__dict__["_pai_log_sink"] = sink           # _training_step_eager logs into it instead of calling self.log
         launches0 = lib.launches
@@ -87,6 +95,8 @@ class StepGraph:
             with torch.cuda.graph(graph):
                 m._training_step_eager((ent.static_x, ent.static_t), batch_idx)
         finally:
+            if gc_enabled:
+                gc.enable()
             m.__dict__.pop("_pai_log_sink", None)
         ent.launches = lib.launches - launches0
         lib.launches = launches0                     # nothing ran during capture
