@@ -15,7 +15,8 @@
 //
 // Tile: M = 128 pixels (TMEM lanes), N = n_tile channels (TMEM columns), K-block = 64 channels
 // (one SWIZZLE_128B row).  Warp roles: 0 = TMA producer, 1 = MMA issuer, 2 = TMEM allocator,
-// 4..7 = epilogue (TMEM -> registers -> global).
+// 4..11 (fprop; 4..7 wgrad) = epilogue (TMEM -> registers -> global; fprop bf16 tiles through a shared-memory box and a
+// TMA store).
 #include <stdio.h>
 #include <stdlib.h>
 
@@ -44,6 +45,7 @@ struct __align__(8) PipeSmem {
     uint64_t empty[kMaxStages];
     uint64_t acc_full[2];
     uint64_t acc_empty[2];
+    uint64_t mask_full[8];        // fprop, masked: per epilogue warp, its TMA load of saved activations has landed
     uint32_t tmem_base;
 };
 
@@ -61,11 +63,13 @@ struct __align__(8) PipeSmem {
 template <bool PAIR, bool MASKED>
 __global__ void __launch_bounds__(kFpropThreads, 1)
 igemm_fprop_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
-                   const IgemmFpropParams p) {
+                   const __grid_constant__ IgemmOutMaps om, const IgemmFpropParams p) {
     pdl_launch_dependents();
     extern __shared__ uint8_t smem_raw[];
     __shared__ PipeSmem ps;
-    __shared__ uint4 stage_buf[8][32 * 8];   // per epilogue warp: 32 rows x 128 B, XOR-swizzled 16-byte chunks
+    // per epilogue warp: 32 rows x 128 B in the SWIZZLE_128B layout (16-byte chunk c of row r at c ^ (r & 7)), the source
+    // box of its TMA stores (and the destination of its TMA loads of saved activations)
+    __shared__ __align__(1024) uint4 stage_buf[8][32 * 8];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -102,6 +106,8 @@ igemm_fprop_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_consta
             mbar_init(&ps.acc_full[a], 1);
             mbar_init(&ps.acc_empty[a], PAIR ? 16 : 8);       // one arrival per epilogue warp (and CTA)
         }
+        if (MASKED)
+            for (int w = 0; w < 8; ++w) mbar_init(&ps.mask_full[w], 1);
         mbar_fence_init();
     }
     if (warp == 2) {
@@ -364,22 +370,19 @@ igemm_fprop_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_consta
         const int q = warp & 3;
         const int half = (warp - 4) >> 2;
         const int r = q * 32 + lane;
-        const int wi = r % p.bw;
-        const int hi = (r / p.bw) % p.bh;
-        const int ni = r / (p.bw * p.bh);
+        // this lane's row (TMEM lane r) inside the pixel box, packed w | h << 8 | n << 16 (each < 128): six separate
+        // position registers, live across the whole tile loop, made the epilogue spill at the 168-register cap
+        const int rpos = (r % p.bw) | (((r / p.bw) % p.bh) << 8) | ((r / (p.bw * p.bh)) << 16);
         const int n_out = p.out2 != nullptr ? 2 : 1;
-        // Rows this lane STORES on the coalesced path: row i * 4 + lane / 8 of the warp's 32, chunk lane % 8.  Their
-        // position inside the pixel box is packed once (w | h << 8 | n << 16); the per-tile offset is plain integer
-        // arithmetic -- the earlier form fetched offset and validity of every stored row with three shuffles, and the
-        // shuffles / shared-memory loads of the epilogue are what slows the main loop (they share the MIO pipe with
-        // the barrier traffic of the producer and MMA warps: without them the N <= 128 layers run 20-40 % faster).
-        int spack[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            const int rs = q * 32 + i * 4 + (lane >> 3);
-            spack[i] = (rs % p.bw) | (((rs / p.bw) % p.bh) << 8) | ((rs / (p.bw * p.bh)) << 16);
-        }
-        // BatchNorm / bias-gradient column sums: this lane's 8 channels (chunk lane % 8) of the rows it stores, carried
+        // The warp's 32 rows are one box of the pixel grid (rows run w-fastest over the power-of-two bw x bh x bn tile box):
+        // its corner inside the tile box is lane 0's row position.  The bf16 path writes a 64-channel chunk of them with ONE TMA store of the
+        // staging tile -- per-lane shared-memory reads and global stores share the MIO pipe with the barrier traffic of
+        // the producer and MMA warps, and slowed the main loop (profiles/r2_igemm_ablation.txt) -- and the TMA clips the
+        // rows and channels outside the output.
+        const int qpos = __shfl_sync(0xffffffffu, rpos, 0);
+        uint4* tile = stage_buf[warp - 4];
+        uint32_t mask_phase = 0;
+        // BatchNorm / bias-gradient column sums: this lane's 8 channels (chunk lane % 8) of rows i * 4 + lane / 8, carried
         // in registers ACROSS tiles and reduced over the 4 row groups + added to the CTA's partial row only when the
         // warp moves to other columns or runs out of tiles (before: 32 shared-memory loads and 4 reductions per chunk)
         // (only where the warp stays on ONE 64-channel block -- N <= 128 or the phase-fused tiles; elsewhere the chunk's
@@ -424,32 +427,29 @@ igemm_fprop_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_consta
             p.fd_tiles_w.divmod(mt, mt, tw);
             p.fd_tiles_h.divmod(mt, tn, th);
             const int col0 = nt * n_tile;
-            const int gw = tw * p.bw + wi, gh = th * p.bh + hi, gn = tn * p.bn + ni;
+            const int gw = tw * p.bw + (rpos & 255), gh = th * p.bh + ((rpos >> 8) & 255), gn = tn * p.bn + (rpos >> 16);
             const bool row_ok = (gw < p.gw) && (gh < p.gh) && (gn < p.gn);
-            const long long off = p.out_phase_off[phase_idx] + (long long)gn * p.out_sn + (long long)gh * p.out_sh +
-                                  (long long)gw * p.out_sw + col0;
-            const long long off2 = (long long)gn * p.out2_sn + (long long)gh * p.out2_sh + (long long)gw * p.out2_sw + col0;
             const int a = it & 1;
             const uint32_t acc_phase = (it >> 1) & 1;
-            const bool vec_ok = ((p.cout & 7) == 0) && ((off & 7) == 0) && ((off2 & 7) == 0);
-            const bool all_vec = __all_sync(0xffffffffu, vec_ok || !row_ok);
-            const bool fast = !p.out_f32 && all_vec && (n_tile & 63) == 0 && col0 + n_tile <= p.cout &&
+            const bool fast = p.tma_out && (n_tile & 63) == 0 && col0 + n_tile <= p.cout &&
                               (p.bias == nullptr || (reinterpret_cast<uintptr_t>(p.bias) & 15) == 0);
             // (the fused-phase mode is only launched when this holds: cout == n_tile == 64, bf16 output)
-            // fused activation backward: the saved activations of this warp's first chunk are fetched while the MMAs of
-            // the tile are still running, those of the next chunk while the current one is packed and stored
+            // the warp's box on the grid
+            const int bw0 = tw * p.bw + (qpos & 255), bh0 = th * p.bh + ((qpos >> 8) & 255), bn0 = tn * p.bn + (qpos >> 16);
+            // fused activation backward: lane 0 TMA-loads the saved activations of the warp's chunk c (the output's box
+            // in the saved tensor; zeros outside it) into the staging tile once the previous store has read it -- the
+            // first chunk while the MMAs of the tile are still running, the next one behind the current chunk's store
             const bool masked = MASKED && p.mask_src != nullptr && fast;   // (MASKED: the instantiation of pai_conv4x4_dgrad_act)
-            // two chunk buffers: both of this warp's chunks of a 256-column (phase-fused) tile are in flight before the
-            // accumulator is waited for -- a DRAM round trip is longer than packing and storing one chunk
-            uint4 mreg[1][8];   // ONE chunk of masks in flight (two cost 32 more registers: every variant of the lean store / statistics path spilled)
-            auto mask_fetch = [&](int c, uint4 (&dst)[8]) {
-                const long long coff = fused ? p.out_phase_off[c >> 6] : 0;
-                const __nv_bfloat16* mrow = reinterpret_cast<const __nv_bfloat16*>(p.mask_src) + off + coff + (fused ? 0 : c);
-#pragma unroll
-                for (int ch = 0; ch < 8; ++ch)
-                    dst[ch] = row_ok ? __ldg(reinterpret_cast<const uint4*>(mrow) + ch) : make_uint4(0, 0, 0, 0);
+            auto mask_load = [&](int c) {
+                __syncwarp();                   // every lane is done reading the tile
+                if (lane == 0) {
+                    bulk_wait_group_read0();
+                    mbar_expect_tx(&ps.mask_full[warp - 4], 32 * 128);
+                    tma_load_4d(tile, &om.aux[fused ? c >> 6 : phase_idx], &ps.mask_full[warp - 4], col0 + (fused ? 0 : c),
+                                bw0, bh0, bn0);
+                }
             };
-            if (masked && 64 * half < acc_n) mask_fetch(64 * half, mreg[0]);
+            if (masked && 64 * half < acc_n) mask_load(64 * half);
             {
                 ROLE_T0();
                 mbar_wait(&ps.acc_full[a], acc_phase);
@@ -475,15 +475,15 @@ igemm_fprop_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_consta
                 released = true;
             };
             if (fast) {
-                // ---- coalesced path: 64 channels of 32 rows are transposed through a swizzled smem tile so
-                // that 8 lanes write one full 128-byte row segment (4 rows per store instruction)
-                uint4* tile = stage_buf[warp - 4];
+                // ---- bf16 path: 64 channels of the warp's 32 rows are packed into the swizzled staging tile, which one
+                // TMA store writes out; lane 0 issues every store of the warp and owns its bulk async-groups
+                // rows of the tile inside the output grid, for the column sums (bit i: row i of the warp's 32)
+                const uint32_t rows_ok = __ballot_sync(0xffffffffu, row_ok);
                 int item = 0;
                 const int n_items = (acc_n >> 6) * n_out;
                 const int last_item = ((n_items - 1) & 1) == half ? n_items - 1 : n_items - 2;   // of this warp (< 0: none)
                 for (int c = 0; c < acc_n; c += 64) {
-                    // fused phases: chunk c is phase c/64 of the same 64 output channels
-                    const long long coff = fused ? p.out_phase_off[c >> 6] : 0;
+                    // fused phases: chunk c is phase (column block) c/64 of the same 64 output channels
                     const int oc = fused ? 0 : c;
                     for (int which = 0; which < n_out; ++which, ++item) {
                         if ((item & 1) != half) continue;
@@ -493,81 +493,74 @@ igemm_fprop_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_consta
                             tmem_ld_16(tmem_d + (uint32_t)(c + 16 * j), *reinterpret_cast<uint32_t(*)[16]>(&v[16 * j]));
                         tmem_ld_wait();
                         if (item == last_item) release_acc();
-                        __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(which == 0 ? p.out : p.out2);
                         const int act = which == 0 ? p.act : p.act2;
-                        const long long my_off = which == 0 ? off : off2;
                         const float* bias_c = p.bias != nullptr ? p.bias + col0 + oc : nullptr;
-                        // activation / bias dispatch hoisted out of the 64-element loop
-                        if (masked && which == 0) {
-                            // this warp's chunks are c = 64 * half + 128 * k (n_out == 1): buffer k & 1
-                            // this warp's chunks are c = 64 * half + 128 * k (n_out == 1): buffer k & 1
-                            mask_pack(v, mreg[0], p.mask_slope, tile, lane);
-                            if (c + 128 < acc_n) mask_fetch(c + 128, mreg[0]);    // next chunk of this warp, behind this one's stores
-                        } else if (act == PAI_ACT_LEAKY)
-                            bias_act_pack<PAI_ACT_LEAKY>(v, bias_c, p.slope, tile, lane);
-                        else if (act == PAI_ACT_RELU)
-                            bias_act_pack<PAI_ACT_RELU>(v, bias_c, p.slope, tile, lane);
-                        else if (act == PAI_ACT_TANH)
-                            bias_act_pack<PAI_ACT_TANH>(v, bias_c, p.slope, tile, lane);
-                        else
-                            bias_act_pack<PAI_ACT_NONE>(v, bias_c, p.slope, tile, lane);
-                        __syncwarp();
-                        const bool stats = p.bn_part != nullptr && which == 0;
-                        if (stats && st_persist && st_col != col0 + oc) {
-                            flush_stats();
-                            st_col = col0 + oc;
+                        if (masked) {
+                            mbar_wait(&ps.mask_full[warp - 4], mask_phase);
+                            mask_phase ^= 1;
+                            mask_pack(v, p.mask_slope, tile, lane);
+                        } else {
+                            if (lane == 0) bulk_wait_group_read0();     // the previous store has read the tile
+                            __syncwarp();
+                            // activation / bias dispatch hoisted out of the 64-element loop
+                            if (act == PAI_ACT_LEAKY)
+                                bias_act_pack<PAI_ACT_LEAKY>(v, bias_c, p.slope, tile, lane);
+                            else if (act == PAI_ACT_RELU)
+                                bias_act_pack<PAI_ACT_RELU>(v, bias_c, p.slope, tile, lane);
+                            else if (act == PAI_ACT_TANH)
+                                bias_act_pack<PAI_ACT_TANH>(v, bias_c, p.slope, tile, lane);
+                            else
+                                bias_act_pack<PAI_ACT_NONE>(v, bias_c, p.slope, tile, lane);
                         }
-                        if (which == 0) {
-                            float cs[8], cq[8];            // this chunk's column sums (8 channels of this lane's rows)
+                        fence_proxy_async_smem();
+                        __syncwarp();
+                        if (lane == 0) {
+                            tma_store_4d(which == 0 ? &om.out[fused ? c >> 6 : phase_idx] : &om.aux[0], tile, col0 + oc,
+                                         bw0, bh0, bn0);
+                            bulk_commit_group();
+                        }
+                        const bool stats = p.bn_part != nullptr && which == 0;
+                        if (stats) {
+                            if (st_persist && st_col != col0 + oc) {
+                                flush_stats();
+                                st_col = col0 + oc;
+                            }
+                            // this chunk's column sums over the rows inside the grid: exactly the stored bf16 values
+                            float cs[8], cq[8];
 #pragma unroll
                             for (int j = 0; j < 8; ++j) cs[j] = cq[j] = 0.f;
-                            const long long tile_off = p.out_phase_off[phase_idx] + coff + col0 + oc + (lane & 7) * 8;
 #pragma unroll
                             for (int i = 0; i < 8; ++i) {
                                 const int row = i * 4 + (lane >> 3), ch = lane & 7;
-                                const int sw_ = tw * p.bw + (spack[i] & 255), sh_ = th * p.bh + ((spack[i] >> 8) & 255);
-                                const int sn_ = tn * p.bn + (spack[i] >> 16);
-                                if (sw_ < p.gw && sh_ < p.gh && sn_ < p.gn) {
+                                if ((rows_ok >> row) & 1u) {
                                     const uint4 val = tile[row * 8 + (ch ^ (row & 7))];
-                                    if (stats) {       // exactly the stored bf16 values
-                                        const __nv_bfloat162* hv = reinterpret_cast<const __nv_bfloat162*>(&val);
+                                    const __nv_bfloat162* hv = reinterpret_cast<const __nv_bfloat162*>(&val);
 #pragma unroll
-                                        for (int j = 0; j < 4; ++j) {
-                                            const float2 f = __bfloat1622float2(hv[j]);
-                                            cs[2 * j] += f.x;
-                                            cs[2 * j + 1] += f.y;
-                                            cq[2 * j] = fmaf(f.x, f.x, cq[2 * j]);
-                                            cq[2 * j + 1] = fmaf(f.y, f.y, cq[2 * j + 1]);
-                                        }
+                                    for (int j = 0; j < 4; ++j) {
+                                        const float2 f = __bfloat1622float2(hv[j]);
+                                        cs[2 * j] += f.x;
+                                        cs[2 * j + 1] += f.y;
+                                        cq[2 * j] = fmaf(f.x, f.x, cq[2 * j]);
+                                        cq[2 * j + 1] = fmaf(f.y, f.y, cq[2 * j + 1]);
                                     }
-                                    *reinterpret_cast<uint4*>(dst + tile_off + (long long)sn_ * p.out_sn + (long long)sh_ * p.out_sh +
-                                                              (long long)sw_ * p.out_sw) = val;
                                 }
                             }
-                            if (stats) {
-                                if (st_persist) {
+                            if (st_persist) {
 #pragma unroll
-                                    for (int j = 0; j < 8; ++j) st_sum[j] += cs[j], st_sq[j] += cq[j];
-                                } else {
-                                    reduce_add(cs, cq, col0 + oc);
-                                }
-                            }
-                        } else {
-                            // second output (its own strides): offsets of the stored rows by shuffle
-#pragma unroll
-                            for (int i = 0; i < 8; ++i) {
-                                const int row = i * 4 + (lane >> 3), ch = lane & 7;
-                                const uint4 val = tile[row * 8 + (ch ^ (row & 7))];
-                                const long long roff = __shfl_sync(0xffffffffu, my_off, row);
-                                const int rok = __shfl_sync(0xffffffffu, (int)row_ok, row);
-                                if (rok) *reinterpret_cast<uint4*>(dst + roff + coff + oc + ch * 8) = val;
+                                for (int j = 0; j < 8; ++j) st_sum[j] += cs[j], st_sq[j] += cq[j];
+                            } else {
+                                reduce_add(cs, cq, col0 + oc);
                             }
                         }
-                                            __syncwarp();
+                        if (masked && c + 128 < acc_n) mask_load(c + 128);   // this warp's next chunk
                     }
                 }
             } else {
-                // ---- generic path (fp32 output, narrow or ragged tiles, split-K accumulation)
+                // ---- generic path (fp32 output, narrow or ragged tiles, split-K accumulation, unaligned bf16 rows)
+                const long long off = p.out_phase_off[phase_idx] + (long long)gn * p.out_sn + (long long)gh * p.out_sh +
+                                      (long long)gw * p.out_sw + col0;
+                const long long off2 = (long long)gn * p.out2_sn + (long long)gh * p.out2_sh + (long long)gw * p.out2_sw + col0;
+                const bool vec_ok = ((p.cout & 7) == 0) && ((off & 7) == 0) && ((off2 & 7) == 0);
                 int step = 0;
                 for (int cc = 0; cc < n_tile; cc += 16, ++step) {
                     if ((step & 1) != half) continue;
@@ -619,6 +612,7 @@ igemm_fprop_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_consta
 #endif
         }
         if (p.bn_part != nullptr) flush_stats();
+        if (lane == 0) bulk_wait_group0();      // the output is written before the CTA exits (and dependents launch)
 #ifdef PAI_PROFILE_ROLES
         if (blockIdx.x == 0 && threadIdx.x == 128)
             printf("[roles] epilogue warp 4: waiting for a full accumulator %lld cyc, working %lld cyc over %d tiles\n", prof_wait, prof_total, it);
@@ -823,8 +817,8 @@ bool igemm_fprop_use_pair(int n_tile, long long m_tiles, int n_tiles, int phases
     return ((m_tiles + 1) / 2) * n_tiles * phases >= 74;
 }
 
-int launch_igemm_fprop(const CUtensorMap& tm_a, const CUtensorMap& tm_b, IgemmFpropParams p, int m_tiles,
-                       int n_tiles, int phases, cudaStream_t stream) {
+int launch_igemm_fprop(const CUtensorMap& tm_a, const CUtensorMap& tm_b, const IgemmOutMaps& om, IgemmFpropParams p,
+                       int m_tiles, int n_tiles, int phases, cudaStream_t stream) {
     const bool pair = p.pair != 0;
     const size_t sub_bytes = 128 * 128 + (size_t)(p.fused_phases ? 4 : 1) * (pair ? p.n_tile / 2 : p.n_tile) * 128;
     if (p.kmma <= 0 || p.kmma > 4) p.kmma = 4;
@@ -880,9 +874,9 @@ int launch_igemm_fprop(const CUtensorMap& tm_a, const CUtensorMap& tm_b, IgemmFp
     if (p.mask_src != nullptr)
         PAI_REQUIRE(!p.out_f32 && p.splitk == 1 && !p.accumulate && (p.n_tile & 63) == 0 && p.cout % p.n_tile == 0 &&
                         (p.cout & 7) == 0 && p.bias == nullptr && p.act == PAI_ACT_NONE && p.out2 == nullptr &&
-                        (reinterpret_cast<uintptr_t>(p.mask_src) & 15) == 0 && (reinterpret_cast<uintptr_t>(p.out) & 15) == 0,
-                    "igemm fprop: the fused activation backward needs a plain bf16 output with cout %% 64 == 0 and no "
-                    "split-K (cout=%d n_tile=%d splitk=%d)", p.cout, p.n_tile, p.splitk);
+                        (reinterpret_cast<uintptr_t>(p.mask_src) & 15) == 0 && p.tma_out,
+                    "igemm fprop: the fused activation backward needs a plain bf16 output with 16 B aligned rows, "
+                    "cout %% 64 == 0 and no split-K (cout=%d n_tile=%d splitk=%d)", p.cout, p.n_tile, p.splitk);
     if (p.bn_part != nullptr) {
         // the statistics ride on the coalesced bf16 epilogue: whole 64-channel chunks, one output, no split-K
         PAI_REQUIRE(!p.out_f32 && p.splitk == 1 && !p.accumulate && (p.n_tile & 63) == 0 && p.cout % p.n_tile == 0 &&
@@ -893,13 +887,13 @@ int launch_igemm_fprop(const CUtensorMap& tm_a, const CUtensorMap& tm_b, IgemmFp
     const int cl = pair ? 2 : 1;
     const dim3 g((unsigned)grid), b(kFpropThreads);
     if (pair && p.mask_src != nullptr)
-        PAI_CUDA_OK(launch_pdl(igemm_fprop_kernel<true, true>, g, b, smem, stream, cl, tm_a, tm_b, p));
+        PAI_CUDA_OK(launch_pdl(igemm_fprop_kernel<true, true>, g, b, smem, stream, cl, tm_a, tm_b, om, p));
     else if (pair)
-        PAI_CUDA_OK(launch_pdl(igemm_fprop_kernel<true, false>, g, b, smem, stream, cl, tm_a, tm_b, p));
+        PAI_CUDA_OK(launch_pdl(igemm_fprop_kernel<true, false>, g, b, smem, stream, cl, tm_a, tm_b, om, p));
     else if (p.mask_src != nullptr)
-        PAI_CUDA_OK(launch_pdl(igemm_fprop_kernel<false, true>, g, b, smem, stream, cl, tm_a, tm_b, p));
+        PAI_CUDA_OK(launch_pdl(igemm_fprop_kernel<false, true>, g, b, smem, stream, cl, tm_a, tm_b, om, p));
     else
-        PAI_CUDA_OK(launch_pdl(igemm_fprop_kernel<false, false>, g, b, smem, stream, cl, tm_a, tm_b, p));
+        PAI_CUDA_OK(launch_pdl(igemm_fprop_kernel<false, false>, g, b, smem, stream, cl, tm_a, tm_b, om, p));
     PAI_CUDA_OK(cudaGetLastError());
     return 0;
 }

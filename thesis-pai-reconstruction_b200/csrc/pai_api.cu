@@ -145,6 +145,48 @@ static const int kTd[2][2] = {{0, -1}, {1, 0}};
 
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
+// 4-D (C, W, H, N) view of a bf16 tensor on the output pixel grid of an igemm fprop launch (element strides sw, sh, sn),
+// box = the 32 accumulator rows of one epilogue warp x 64 channels.  The 128 rows of a tile run w-fastest over the
+// power-of-two bw x bh x bn pixel box, so a warp's 32 rows are always the box {64, min(bw, 32), ...}.
+static int map_out(CUtensorMap* m, const void* base, int cout, int gw, int gh, int gn, long long sw, long long sh,
+                   long long sn, const PixBox& b) {
+    const int bw = b.bw < 32 ? b.bw : 32, bh = b.bh < 32 / bw ? b.bh : 32 / bw, bn = 32 / (bw * bh);
+    // a size-1 H dimension may have stride 0 (pointwise rows); TMA wants a non-zero multiple of 16 bytes
+    if (sh == 0) sh = (long long)gw * sw;
+    uint64_t dims[4] = {(uint64_t)cout, (uint64_t)gw, (uint64_t)gh, (uint64_t)gn};
+    uint64_t str[3] = {(uint64_t)sw * 2, (uint64_t)sh * 2, (uint64_t)sn * 2};
+    uint32_t box[4] = {64, (uint32_t)bw, (uint32_t)bh, (uint32_t)bn};
+    return encode_tmap_bf16(m, base, 4, dims, str, box);
+}
+
+// Output maps of a launch (IgemmOutMaps) for `nmaps` phases / column blocks of p.out, from the strides and phase offsets
+// already in `p` (and maps of p.out2 or p.mask_src).  Without 16-byte aligned bf16 rows there are none and every tile
+// takes the generic epilogue (p.tma_out stays 0).
+static int map_outputs(IgemmOutMaps* om, IgemmFpropParams& p, int nmaps, const PixBox& b) {
+    p.tma_out = 0;
+    const bool ok = !p.out_f32 && !p.accumulate && (p.cout & 7) == 0 && aligned16(p.out) && p.out_sw % 8 == 0 &&
+                    p.out_sh % 8 == 0 && p.out_sn % 8 == 0 &&
+                    (p.out2 == nullptr || (aligned16(p.out2) && p.out2_sw % 8 == 0 && p.out2_sh % 8 == 0 && p.out2_sn % 8 == 0));
+    if (!ok) return 0;
+    for (int j = 0; j < nmaps; ++j) {
+        PAI_REQUIRE(p.out_phase_off[j] % 8 == 0, "igemm fprop: phase offset %lld is not 16 B aligned", p.out_phase_off[j]);
+        int rc = map_out(&om->out[j], static_cast<const __nv_bfloat16*>(p.out) + p.out_phase_off[j], p.cout, p.gw, p.gh,
+                         p.gn, p.out_sw, p.out_sh, p.out_sn, b);
+        if (rc) return rc;
+        if (p.mask_src != nullptr) {
+            rc = map_out(&om->aux[j], static_cast<const __nv_bfloat16*>(p.mask_src) + p.out_phase_off[j], p.cout, p.gw,
+                         p.gh, p.gn, p.out_sw, p.out_sh, p.out_sn, b);
+            if (rc) return rc;
+        }
+    }
+    if (p.out2 != nullptr) {
+        int rc = map_out(&om->aux[0], p.out2, p.cout, p.gw, p.gh, p.gn, p.out2_sw, p.out2_sh, p.out2_sn, b);
+        if (rc) return rc;
+    }
+    p.tma_out = 1;
+    return 0;
+}
+
 // Output-channel tile: the widest of 256/128/64/32/16 that divides cout_pad while still giving every
 // SM a tile (wider tiles re-read the activations less often from L2).
 static int auto_n_tile(int cout_pad, long long m_tiles_x_phases) {
@@ -222,6 +264,8 @@ static int conv4x4_fprop_impl(const void* x, int n, int h, int w, int cin, int x
 
     IgemmFpropParams p;
     memset(&p, 0, sizeof(p));
+    IgemmOutMaps om;
+    memset(&om, 0, sizeof(om));
     p.pair = pair;
     p.bw = b.bw, p.bh = b.bh, p.bn = b.bn, p.tiles_w = b.tiles_w, p.tiles_h = b.tiles_h;
     p.gw = wo, p.gh = ho, p.gn = n;
@@ -244,7 +288,7 @@ static int conv4x4_fprop_impl(const void* x, int n, int h, int w, int cin, int x
     if (p.splitk > 1) {
         p.out_sn = (long long)ho * wo * cout, p.out_sh = (long long)wo * cout, p.out_sw = cout;
         p.out_f32 = 1, p.accumulate = 1, p.out = splitk_ws;
-        int rc2 = launch_igemm_fprop(tm_a, tm_b, p, m_tiles, cout_pad / n_tile, 1, (cudaStream_t)stream);
+        int rc2 = launch_igemm_fprop(tm_a, tm_b, om, p, m_tiles, cout_pad / n_tile, 1, (cudaStream_t)stream);
         if (rc2) return rc2;
         return launch_splitk_finish(splitk_ws, (long long)n * ho * wo, cout, bias, act, slope, y, y_ld, y_f32,
                                     (cudaStream_t)stream);
@@ -257,7 +301,9 @@ static int conv4x4_fprop_impl(const void* x, int n, int h, int w, int cin, int x
         p.out2 = y2, p.act2 = act2;
         p.out2_sn = (long long)ho * wo * y2_ld, p.out2_sh = (long long)wo * y2_ld, p.out2_sw = y2_ld;
     }
-    return launch_igemm_fprop(tm_a, tm_b, p, m_tiles, cout_pad / n_tile, 1, (cudaStream_t)stream);
+    rc = map_outputs(&om, p, 1, b);
+    if (rc) return rc;
+    return launch_igemm_fprop(tm_a, tm_b, om, p, m_tiles, cout_pad / n_tile, 1, (cudaStream_t)stream);
 }
 
 int pai_conv4x4_fprop_dual(const void* x, int n, int h, int w, int cin, int x_ld, const void* w_packed, int cout,
@@ -314,6 +360,8 @@ static int convT4x4s2_fprop_impl(const void* x, int n, int h, int w, int cin, in
 
     IgemmFpropParams p;
     memset(&p, 0, sizeof(p));
+    IgemmOutMaps om;
+    memset(&om, 0, sizeof(om));
     p.pair = pair;
     p.bw = b.bw, p.bh = b.bh, p.bn = b.bn, p.tiles_w = b.tiles_w, p.tiles_h = b.tiles_h;
     p.gw = w, p.gh = h, p.gn = n;
@@ -365,17 +413,21 @@ static int convT4x4s2_fprop_impl(const void* x, int n, int h, int w, int cin, in
         for (int py = 0; py < 2; ++py)
             for (int px = 0; px < 2; ++px) p.out_phase_off[col_of_phase[py * 2 + px]] = (py * wo + px) * ld;
         p.bias = bias, p.act = act, p.slope = slope, p.out_f32 = 0, p.out = y;
-        return launch_igemm_fprop(tm_a, tm_b, p, m_tiles, 1, 1, (cudaStream_t)stream);
+        rc = map_outputs(&om, p, 4, b);
+        if (rc) return rc;
+        return launch_igemm_fprop(tm_a, tm_b, om, p, m_tiles, 1, 1, (cudaStream_t)stream);
     }
     if (p.splitk > 1) {
         p.out_f32 = 1, p.accumulate = 1, p.out = splitk_ws;
-        int rc2 = launch_igemm_fprop(tm_a, tm_b, p, m_tiles, cout_pad / n_tile, 4, (cudaStream_t)stream);
+        int rc2 = launch_igemm_fprop(tm_a, tm_b, om, p, m_tiles, cout_pad / n_tile, 4, (cudaStream_t)stream);
         if (rc2) return rc2;
         return launch_splitk_finish(splitk_ws, 4LL * n * h * w, cout, bias, act, slope, y, y_ld, y_f32,
                                     (cudaStream_t)stream);
     }
     p.bias = bias, p.act = act, p.slope = slope, p.out_f32 = y_f32, p.out = y;
-    return launch_igemm_fprop(tm_a, tm_b, p, m_tiles, cout_pad / n_tile, 4, (cudaStream_t)stream);
+    rc = map_outputs(&om, p, 4, b);
+    if (rc) return rc;
+    return launch_igemm_fprop(tm_a, tm_b, om, p, m_tiles, cout_pad / n_tile, 4, (cudaStream_t)stream);
 }
 
 int pai_convT4x4s2_fprop(const void* x, int n, int h, int w, int cin, int x_ld, const void* w_packed, int cout,
@@ -493,6 +545,8 @@ int pai_pointwise_gemm(const void* x, long long m, int cin, int x_ld, const void
     if (rc) return rc;
     IgemmFpropParams p;
     memset(&p, 0, sizeof(p));
+    IgemmOutMaps om;
+    memset(&om, 0, sizeof(om));
     p.bw = b.bw, p.bh = b.bh, p.bn = b.bn, p.tiles_w = b.tiles_w, p.tiles_h = b.tiles_h;
     p.gw = wbox, p.gh = 1, p.gn = n;
     p.n_tile = n_tile, p.cout = cout, p.kc_per_tap = cin / 64, p.ntaps = 1;
@@ -501,7 +555,9 @@ int pai_pointwise_gemm(const void* x, long long m, int cin, int x_ld, const void
     p.out2_sn = (long long)wbox * y2_ld, p.out2_sh = 0, p.out2_sw = y2_ld;
     p.bias = bias, p.act = act, p.slope = slope, p.out_f32 = y_f32, p.out = y, p.out2 = y2, p.act2 = act2;
     p.kmma = k_valid > 0 ? k_valid / 16 : 4;
-    return launch_igemm_fprop(tm_a, tm_b, p, b.tiles_w * b.tiles_h * b.tiles_n, cout_pad / n_tile, 1,
+    rc = map_outputs(&om, p, 1, b);
+    if (rc) return rc;
+    return launch_igemm_fprop(tm_a, tm_b, om, p, b.tiles_w * b.tiles_h * b.tiles_n, cout_pad / n_tile, 1,
                               (cudaStream_t)stream);
 }
 
@@ -532,6 +588,8 @@ int pai_conv3x3_fprop(const void* x, int n, int h, int w, int cin, int x_ld, con
     if (rc) return rc;
     IgemmFpropParams p;
     memset(&p, 0, sizeof(p));
+    IgemmOutMaps om;
+    memset(&om, 0, sizeof(om));
     p.bw = b.bw, p.bh = b.bh, p.bn = b.bn, p.tiles_w = b.tiles_w, p.tiles_h = b.tiles_h;
     p.gw = w, p.gh = h, p.gn = n;
     p.n_tile = n_tile, p.cout = cout, p.kc_per_tap = cin / 64, p.ntaps = 9;
@@ -542,14 +600,16 @@ int pai_conv3x3_fprop(const void* x, int n, int h, int w, int cin, int x_ld, con
     if (p.splitk > 1) {
         p.out_sn = (long long)h * w * cout, p.out_sh = (long long)w * cout, p.out_sw = cout;
         p.out_f32 = 1, p.accumulate = 1, p.out = splitk_ws;
-        int rc2 = launch_igemm_fprop(tm_a, tm_b, p, m_tiles, cout_pad / n_tile, 1, (cudaStream_t)stream);
+        int rc2 = launch_igemm_fprop(tm_a, tm_b, om, p, m_tiles, cout_pad / n_tile, 1, (cudaStream_t)stream);
         if (rc2) return rc2;
         return launch_splitk_finish(splitk_ws, (long long)n * h * w, cout, bias, act, slope, y, y_ld, y_f32,
                                     (cudaStream_t)stream);
     }
     p.out_sn = (long long)h * w * y_ld, p.out_sh = (long long)w * y_ld, p.out_sw = y_ld;
     p.bias = bias, p.act = act, p.slope = slope, p.out_f32 = y_f32, p.out = y;
-    return launch_igemm_fprop(tm_a, tm_b, p, m_tiles, cout_pad / n_tile, 1, (cudaStream_t)stream);
+    rc = map_outputs(&om, p, 1, b);
+    if (rc) return rc;
+    return launch_igemm_fprop(tm_a, tm_b, om, p, m_tiles, cout_pad / n_tile, 1, (cudaStream_t)stream);
 }
 
 int pai_conv3x3_wgrad(const void* x, int n, int h, int w, int cin, int x_ld, const void* gy, int cout, int gy_ld,

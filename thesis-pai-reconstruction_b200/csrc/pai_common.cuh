@@ -159,6 +159,28 @@ __device__ __forceinline__ void tma_prefetch_5d(const CUtensorMap* map, int c0, 
                  "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
                  : "memory");
 }
+__device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2,
+                                            int c3) {
+    asm volatile(
+        "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
+        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+        : "memory");
+}
+// TMA store of a 4-D box from shared memory (elements outside the map's extents are not written), tracked by the
+// issuing thread's bulk async-groups: commit after the store, then wait_group_read before that thread (and, after a
+// warp sync, its warp) writes the source buffer again, and wait_group before the CTA exits.  The shared-memory writes
+// the store reads must be fenced to the async proxy first (fence_proxy_async_smem in every writing thread).
+__device__ __forceinline__ void tma_store_4d(const CUtensorMap* map, const void* src, int c0, int c1, int c2, int c3) {
+    asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(
+                     reinterpret_cast<uint64_t>(map)),
+                 "r"(smem_u32(src)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+                 : "memory");
+}
+__device__ __forceinline__ void bulk_commit_group() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+// every committed bulk store of this thread has finished READING its shared-memory source
+__device__ __forceinline__ void bulk_wait_group_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
+// every committed bulk store of this thread has completed (its global writes are performed)
+__device__ __forceinline__ void bulk_wait_group0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* map) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(map)) : "memory");
 }

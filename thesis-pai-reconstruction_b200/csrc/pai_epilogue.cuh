@@ -1,5 +1,6 @@
 // Epilogue helpers shared by the tcgen05 kernels (igemm.cu, thin.cu): TMEM accumulator rows -> bias / activation ->
-// bf16 -> XOR-swizzled shared-memory transpose tile -> coalesced 128-byte row segments.
+// bf16 -> XOR-swizzled (SWIZZLE_128B) shared-memory tile -> global memory (a TMA store in igemm.cu, coalesced 128-byte
+// row segments in thin.cu).
 #pragma once
 #include "pai_common.cuh"
 #include "pai_kernels.h"
@@ -76,12 +77,15 @@ __device__ __forceinline__ void bias_act_pack(const uint32_t (&v)[64], const flo
     }
 }
 
-// out = acc * (saved > 0 ? 1 : slope): the activation backward of the layer whose data gradient this GEMM produces;
-// m = this lane's 64 saved activations (zeros for rows outside the tensor), fetched by the caller ahead of time
-__device__ __forceinline__ void mask_pack(const uint32_t (&v)[64], const uint4 (&m)[8], float slope, uint4* tile, int lane) {
+// out = acc * (saved > 0 ? 1 : slope): the activation backward of the layer whose data gradient this GEMM produces.
+// Works in place: the tile already holds this lane's row of 64 saved activations in the same swizzled layout (a TMA
+// load of the output's box from the saved tensor; zeros for rows outside it), and each 16-byte slot is replaced by the
+// product it gates.
+__device__ __forceinline__ void mask_pack(const uint32_t (&v)[64], float slope, uint4* tile, int lane) {
 #pragma unroll
     for (int ch = 0; ch < 8; ++ch) {
-        const __nv_bfloat162* mh = reinterpret_cast<const __nv_bfloat162*>(&m[ch]);
+        const uint4 m = tile[lane * 8 + (ch ^ (lane & 7))];
+        const __nv_bfloat162* mh = reinterpret_cast<const __nv_bfloat162*>(&m);
         uint32_t w[4];
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
@@ -95,20 +99,6 @@ __device__ __forceinline__ void mask_pack(const uint32_t (&v)[64], const uint4 (
     }
 }
 
-
-// Writes the 32 x 64 bf16 transpose tile of one epilogue warp (filled by bias_act_pack / mask_pack) to global memory:
-// 8 lanes store one full 128-byte row segment, 4 rows per instruction.  row_off / row_ok are this lane's own row.
-__device__ __forceinline__ void store_tile_rows(const uint4* tile, __nv_bfloat16* dst, long long row_off, bool row_ok,
-                                                int lane) {
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        const int row = i * 4 + (lane >> 3), ch = lane & 7;
-        const uint4 val = tile[row * 8 + (ch ^ (row & 7))];
-        const long long roff = __shfl_sync(0xffffffffu, row_off, row);
-        const int rok = __shfl_sync(0xffffffffu, (int)row_ok, row);
-        if (rok) *reinterpret_cast<uint4*>(dst + roff + ch * 8) = val;
-    }
-}
 
 // byte offset of 16-byte chunk `c` (0..7) of row `r` inside a SWIZZLE_128B tile with 128-byte rows (tile base aligned to
 // 1024 B): the layout a TMA box with a 64-element bf16 inner dimension writes and the K-major UMMA descriptors read

@@ -82,6 +82,20 @@ struct IgemmFpropParams {
     int pair;                  // run as 2-CTA clusters (cta_group::2, M = 256): tm_b's box must hold n_tile / 2 rows
     int splitk;                // K slices per output tile (>1: partial sums are accumulated into fp32 `out`)
     int accumulate;            // generic fp32 path adds into `out` (red.add) instead of storing
+    // the IgemmOutMaps of the launch describe `out` (and `out2` / `mask_src`): 64-channel chunks of bf16 tiles go out as
+    // TMA stores.  Set by the host only where those maps exist (bf16 output, 16-byte aligned base and rows).
+    int tma_out;
+};
+
+// TMA maps of the bf16 outputs of an igemm fprop launch: 4-D (C, W, H, N) views of `out` + out_phase_off[j] with the
+// output's strides, extents (cout, gw, gh, gn) -- TMA clips ragged pixel tiles and channel tails -- and a box of one
+// epilogue warp's 32 accumulator rows x 64 channels, SWIZZLE_128B (the layout of the warp's staging tile).
+//   out[j]: column block j of a phase-fused tile, phase j otherwise (the index of out_phase_off)
+//   aux[j]: the saved activations of a masked data gradient at the same positions (mask_src + out_phase_off[j]);
+//           or aux[0] = `out2` with its own strides
+struct IgemmOutMaps {
+    CUtensorMap out[4];
+    CUtensorMap aux[4];
 };
 
 struct IgemmWgradParams {
@@ -101,8 +115,8 @@ struct IgemmWgradParams {
 };
 
 bool igemm_fprop_use_pair(int n_tile, long long m_tiles, int n_tiles, int phases, int splitk);
-int launch_igemm_fprop(const CUtensorMap& tm_a, const CUtensorMap& tm_b, IgemmFpropParams p, int m_tiles,
-                       int n_tiles, int phases, cudaStream_t stream);
+int launch_igemm_fprop(const CUtensorMap& tm_a, const CUtensorMap& tm_b, const IgemmOutMaps& om, IgemmFpropParams p,
+                       int m_tiles, int n_tiles, int phases, cudaStream_t stream);
 // y[pix * ld + c] = act(ws[pix * c_count + c] + bias[c]) for a dense fp32 split-K workspace
 int launch_splitk_finish(const float* ws, long long pixels, int cout, const float* bias, int act, float slope, void* y,
                          int y_ld, int y_f32, cudaStream_t stream);
