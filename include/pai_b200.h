@@ -375,6 +375,40 @@ int pai_attn_fwd(const void* qkv, int s, int b, int heads, int head_dim, float* 
 int pai_attn_bwd(const void* qkv, const void* dout, int s, int b, int heads, int head_dim, const float* probs,
                  float* ds_work, void* dqkv, void* stream);
 
+/* Train-mode dropout of nn.TransformerEncoderLayer(d, 8, dropout=p) (torch's TransformerEncoderLayer._sa_block /
+ * _ff_block), fused into the kernels above.  The mask is regenerated from a counter-based RNG (Philox4x32-10) in
+ * every kernel that applies it, forward and backward, and never stored.  Element idx of site `site` under the
+ * 64-bit key *key (a device pointer, so a CUDA graph replay can draw a new key):
+ *   r = word (idx & 3) of philox4x32_10(counter = (lo32(idx >> 2), hi32(idx >> 2), site, 0), key = (lo32, hi32)),
+ *   dropped iff r < llround(p * 2^32) (double precision, clamped to 2^32 - 1); kept elements are scaled by 1/(1-p).
+ * Site = layer * 4 + k; idx is the element's linear index in the tensor of site k:
+ *   k = 0  attention probabilities [b*heads, s, s] (MultiheadAttention's dropout_p)     pai_attn_fwd/bwd_dropout
+ *   k = 1  attention block output [s*b, d] before norm1(x + .) (dropout1)               pai_add_dropout_layernorm_fwd,
+ *   k = 3  feed-forward output [s*b, d] before norm2(x + .) (dropout2)                    pai_layernorm_bwd_dropout
+ *   k = 2  after the GELU, [s*b, dim_feedforward] (dropout)                             pai_gelu_dropout_fwd/bwd
+ * Every entry point rejects a null key and p outside (0, 1) before any CUDA call.
+ *   pai_dropout_mask               out_u8[idx] = 1 (kept) / 0 (dropped), idx < n: the mask the kernels apply
+ *   pai_attn_fwd_dropout           out = (P o M / (1-p)) V; probs keeps the undropped softmax P
+ *   pai_attn_bwd_dropout           dP = (dO V^T) o M / (1-p), dS = P o (dP - rowsum(P o dP)), dV = (P o M / (1-p))^T dO
+ *   pai_add_dropout_layernorm_fwd  z = x + y o M / (1-p) (bf16, saved for the backward), out = LayerNorm(z); d % 4 == 0
+ *   pai_layernorm_bwd_dropout      pai_layernorm_bwd of (z, g) -> dz, dgamma, dbeta, and dy = dz o M / (1-p)
+ *   pai_gelu_dropout_fwd/bwd       y = GELU(x) o M / (1-p);  dx = g o M / (1-p) o GELU'(x); n % 4 == 0
+ */
+int pai_dropout_mask(const long long* key, int site, long long n, float p, void* out_u8, void* stream);
+int pai_attn_fwd_dropout(const void* qkv, int s, int b, int heads, int head_dim, const long long* key, int site, float p,
+                         float* probs, void* out, void* stream);
+int pai_attn_bwd_dropout(const void* qkv, const void* dout, int s, int b, int heads, int head_dim, const long long* key,
+                         int site, float p, const float* probs, float* ds_work, void* dqkv, void* stream);
+int pai_add_dropout_layernorm_fwd(const void* x, const void* y, long long m, int d, const long long* key, int site, float p,
+                                  const float* gamma, const float* beta, float eps, void* z, void* out, float* mean,
+                                  float* rstd, void* stream);
+int pai_layernorm_bwd_dropout(const void* z, const void* g, long long m, int d, const float* gamma, const float* mean,
+                              const float* rstd, const long long* key, int site, float p, void* dz, void* dy,
+                              float* dgamma, float* dbeta, void* stream);
+int pai_gelu_dropout_fwd(const void* x, long long n, const long long* key, int site, float p, void* y, void* stream);
+int pai_gelu_dropout_bwd(const void* x, const void* g, long long n, const long long* key, int site, float p, void* dx,
+                         void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * fp32 check path (north star: "1e-5 with the fp32 accumulate check path").  Slow, exact twins of the tensor-core
  * layers on fp32 NCHW tensors in the reference's own layouts: one thread per output element, fp32 FMA accumulation,

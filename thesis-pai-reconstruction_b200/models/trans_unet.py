@@ -10,6 +10,8 @@ and initial weights are the reference's (the torch modules only hold parameters)
   ``nn.TransformerEncoderLayer``s.  The reference builds them without ``batch_first`` and feeds [n, patches, d], so
   attention runs over the BATCH axis (SURVEY.md Q4) -- reproduced exactly: sequence = images of this GPU's batch.
   Linear layers run on the pointwise GEMM; LayerNorm, GELU and the attention core are kernels of csrc/transformer.cu.
+  Train-mode dropout (the layer's four sites) is fused into those kernels: each forward draws one int64 key from
+  torch's CUDA generator and the kernels regenerate their Philox masks from it (csrc/pai_dropout.cuh).
 * decoders: 2 x (3x3 conv + BN + ReLU) + nearest upsample on the 9-tap implicit GEMM.
 """
 import math
@@ -116,6 +118,7 @@ class VisionTransformer(nn.Module):
         side = int(math.sqrt(num_patches))
         self.to_image = Rearrange("n (h w) (p1 p2 c) -> n c (h p1) (w p2)", h=side, w=side, p1=patch_size, p2=patch_size)
         self.patch_size, self.num_heads, self.dropout = patch_size, num_heads, dropout
+        self._dropout_key = None     # int64 [1] device tensor: the key of the last train-mode forward with dropout
 
     def _layer(self, x, lyr, s, b):
         att = lyr.self_attn
@@ -125,9 +128,26 @@ class VisionTransformer(nn.Module):
         f = L.linear(L.gelu(L.linear(x, lyr.linear1.weight, lyr.linear1.bias)), lyr.linear2.weight, lyr.linear2.bias)
         return L.layernorm(L.add_act(x, f), lyr.norm2)
 
+    def _layer_dropout(self, x, lyr, s, b, key, site):
+        """``_layer`` with the train-mode dropout of nn.TransformerEncoderLayer at sites ``site + 0..3``: attention
+        probabilities, attention output (dropout1), after the GELU (dropout), feed-forward output (dropout2)."""
+        att, p = lyr.self_attn, self.dropout
+        qkv = L.linear(x, att.in_proj_weight, att.in_proj_bias)
+        a = L.attention_dropout(qkv, s, b, self.num_heads, key, site, p)
+        x = L.add_dropout_layernorm(x, L.linear(a, att.out_proj.weight, att.out_proj.bias), lyr.norm1, key, site + 1, p)
+        h = L.gelu_dropout(L.linear(x, lyr.linear1.weight, lyr.linear1.bias), key, site + 2, p)
+        f = L.linear(h, lyr.linear2.weight, lyr.linear2.bias)
+        return L.add_dropout_layernorm(x, f, lyr.norm2, key, site + 3, p)
+
     def forward(self, x):
+        key = None
         if self.training and self.dropout > 0:
-            raise RuntimeError("pai_b200: train-mode dropout > 0 is not implemented on the B200 path; no fallback exists")
+            if self.dropout >= 1:
+                raise RuntimeError(f"pai_b200: ViT dropout must be < 1 in training mode, got {self.dropout}")
+            # one draw from torch's CUDA generator per forward: seeded by torch.manual_seed, and a new key at every
+            # replay of a captured step graph
+            key = torch.randint(-2 ** 63, 2 ** 63 - 1, (1,), dtype=torch.int64, device=x.device)
+            self._dropout_key = key
         n, hh, ww, c = x.shape
         p = self.patch_size
         gh, gw = hh // p, ww // p
@@ -144,8 +164,8 @@ class VisionTransformer(nn.Module):
         t = L.layernorm(t, emb[3])
         t = (t.view(n, tokens, d) + self.pos_embedding.to(t.dtype)).reshape(n * tokens, d)
         # no batch_first in the reference: sequence axis = n (batch), "batch" axis = tokens
-        for lyr in self.transformer.layers:
-            t = self._layer(t, lyr, n, tokens)
+        for i, lyr in enumerate(self.transformer.layers):
+            t = self._layer(t, lyr, n, tokens) if key is None else self._layer_dropout(t, lyr, n, tokens, key, 4 * i)
         return t.view(n, gh, gw, p, p, c).permute(0, 1, 3, 2, 4, 5).reshape(n, hh, ww, c)
 
 

@@ -779,6 +779,57 @@ class _Attention(torch.autograd.Function):
         return ops.attn_bwd(qkv, g.contiguous(), probs, s, b, heads), None, None, None
 
 
+# Train-mode dropout of nn.TransformerEncoderLayer: each node saves the forward's int64 key tensor (never a mask); the
+# backward kernels regenerate the mask of their ``site`` from it.
+class _AttentionDropout(torch.autograd.Function):
+    """softmax(Q K^T / sqrt(hd)) with dropout on the probabilities, times V (site 0 of a layer)."""
+
+    @staticmethod
+    def forward(ctx, qkv, s, b, heads, key, site, p):
+        out, probs = ops.attn_fwd_dropout(qkv, s, b, heads, key, site, p)
+        ctx.save_for_backward(qkv, probs, key)
+        ctx.dims = (s, b, heads, site, p)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        qkv, probs, key = ctx.saved_tensors
+        s, b, heads, site, p = ctx.dims
+        return ops.attn_bwd_dropout(qkv, g.contiguous(), probs, s, b, heads, key, site, p), None, None, None, None, None, None
+
+
+class _AddDropoutLayerNorm(torch.autograd.Function):
+    """LayerNorm(x + dropout(y)): the residual add and norm after the attention (site 1) or feed-forward (site 3) block."""
+
+    @staticmethod
+    def forward(ctx, x, y, weight, bias, eps, key, site, p):
+        z, out, mean, rstd = ops.add_dropout_layernorm_fwd(x, y, weight.detach(), bias.detach(), eps, key, site, p)
+        ctx.save_for_backward(z, weight, mean, rstd, key)
+        ctx.site, ctx.p = site, p
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        z, weight, mean, rstd, key = ctx.saved_tensors
+        dz, dy, dgamma, dbeta = ops.layernorm_bwd_dropout(z, g.contiguous(), weight.detach(), mean, rstd, key, ctx.site, ctx.p)
+        return dz, dy, dgamma, dbeta, None, None, None, None
+
+
+class _GeluDropout(torch.autograd.Function):
+    """dropout(GELU(x)) inside the feed-forward block (site 2)."""
+
+    @staticmethod
+    def forward(ctx, x, key, site, p):
+        ctx.save_for_backward(x, key)
+        ctx.site, ctx.p = site, p
+        return ops.gelu_dropout_fwd(x, key, site, p)
+
+    @staticmethod
+    def backward(ctx, g):
+        x, key = ctx.saved_tensors
+        return ops.gelu_dropout_bwd(x, g.contiguous(), key, ctx.site, ctx.p), None, None, None
+
+
 def conv1x1_padded(x, mod: nn.Conv2d):
     if mod.bias is not None or mod.kernel_size != (1, 1) or mod.groups != 1 or x.shape[-1] != _pad64(mod.in_channels):
         raise RuntimeError(f"pai_b200: unexpected bottleneck projection {mod}")
@@ -813,6 +864,18 @@ def gelu(x2d):
 
 def attention(qkv2d, s, b, heads):
     return _Attention.apply(qkv2d, s, b, heads)
+
+
+def attention_dropout(qkv2d, s, b, heads, key, site, p):
+    return _AttentionDropout.apply(qkv2d, s, b, heads, key, site, p)
+
+
+def add_dropout_layernorm(x2d, y2d, mod: nn.LayerNorm, key, site, p):
+    return _AddDropoutLayerNorm.apply(x2d, y2d, mod.weight, mod.bias, mod.eps, key, site, p)
+
+
+def gelu_dropout(x2d, key, site, p):
+    return _GeluDropout.apply(x2d, key, site, p)
 
 
 def to_plane(x: torch.Tensor) -> torch.Tensor:

@@ -82,6 +82,16 @@ SIGNATURES = {
     "pai_gelu_bwd": [c_void_p, c_void_p, c_ll, c_void_p, c_void_p],
     "pai_attn_fwd": [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p],
     "pai_attn_bwd": [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p],
+    "pai_dropout_mask": [c_void_p, c_int, c_ll, c_float, c_void_p, c_void_p],
+    "pai_attn_fwd_dropout": [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_float, c_void_p, c_void_p, c_void_p],
+    "pai_attn_bwd_dropout": [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_float, c_void_p, c_void_p,
+                             c_void_p, c_void_p],
+    "pai_add_dropout_layernorm_fwd": [c_void_p, c_void_p, c_ll, c_int, c_void_p, c_int, c_float, c_void_p, c_void_p,
+                                      c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
+    "pai_layernorm_bwd_dropout": [c_void_p, c_void_p, c_ll, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_float,
+                                  c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
+    "pai_gelu_dropout_fwd": [c_void_p, c_ll, c_void_p, c_int, c_float, c_void_p, c_void_p],
+    "pai_gelu_dropout_bwd": [c_void_p, c_void_p, c_ll, c_void_p, c_int, c_float, c_void_p, c_void_p],
     "pai_adam_pack_conv4x4": [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_float, c_float, c_float, c_float,
                               c_float, c_void_p, c_void_p, c_int, c_void_p, c_void_p],
     "pai_scale_channels": [c_void_p, c_int, c_void_p, c_int, c_ll, c_int, c_void_p, c_int, c_void_p],

@@ -804,6 +804,73 @@ def attn_bwd(qkv, dout, probs, s, b, heads):
     return dqkv
 
 
+# Train-mode dropout of the encoder layer (csrc/pai_dropout.cuh): ``key`` is a one-element int64 device tensor, the
+# masks are regenerated from (element index, site, key) inside the kernels and never stored.
+def _key(key):
+    assert key.dtype == torch.int64 and key.numel() == 1 and key.is_cuda
+    return _ptr(key)
+
+
+def dropout_mask(key, site, n, p):
+    """uint8 ``[n]``: 1 where the fused kernels keep element ``i`` of ``site``, 0 where they drop it."""
+    out = torch.empty(n, dtype=torch.uint8, device=key.device)
+    lib.call("pai_dropout_mask", _key(key), site, n, float(p), _ptr(out), _stream())
+    return out
+
+
+def attn_fwd_dropout(qkv, s, b, heads, key, site, p):
+    e = qkv.shape[1] // 3
+    probs = torch.empty(b * heads, s, s, dtype=torch.float32, device=qkv.device)
+    out = torch.empty(s * b, e, dtype=torch.bfloat16, device=qkv.device)
+    lib.call("pai_attn_fwd_dropout", _ptr(qkv), s, b, heads, e // heads, _key(key), site, float(p), _ptr(probs), _ptr(out),
+             _stream())
+    return out, probs
+
+
+def attn_bwd_dropout(qkv, dout, probs, s, b, heads, key, site, p):
+    e = qkv.shape[1] // 3
+    work = torch.empty_like(probs)
+    dqkv = torch.empty_like(qkv)
+    lib.call("pai_attn_bwd_dropout", _ptr(qkv), _ptr(dout), s, b, heads, e // heads, _key(key), site, float(p), _ptr(probs),
+             _ptr(work), _ptr(dqkv), _stream(), kernels=2)
+    return dqkv
+
+
+def add_dropout_layernorm_fwd(x, y, gamma, beta, eps, key, site, p):
+    """-> (z = x + dropout(y), LayerNorm(z), mean, rstd)."""
+    m, d = x.shape
+    assert y.shape == x.shape and x.is_contiguous() and y.is_contiguous()
+    z, out = torch.empty_like(x), torch.empty_like(x)
+    mean = torch.empty(m, dtype=torch.float32, device=x.device)
+    rstd = torch.empty(m, dtype=torch.float32, device=x.device)
+    lib.call("pai_add_dropout_layernorm_fwd", _ptr(x), _ptr(y), m, d, _key(key), site, float(p), _ptr(gamma), _ptr(beta),
+             float(eps), _ptr(z), _ptr(out), _ptr(mean), _ptr(rstd), _stream())
+    return z, out, mean, rstd
+
+
+def layernorm_bwd_dropout(z, g, gamma, mean, rstd, key, site, p):
+    """-> (dz, dy, dgamma, dbeta): the residual branch's and the dropout branch's gradients."""
+    m, d = z.shape
+    dz, dy = torch.empty_like(z), torch.empty_like(z)
+    dgamma = torch.empty(d, dtype=torch.float32, device=z.device)
+    dbeta = torch.empty(d, dtype=torch.float32, device=z.device)
+    lib.call("pai_layernorm_bwd_dropout", _ptr(z), _ptr(g), m, d, _ptr(gamma), _ptr(mean), _ptr(rstd), _key(key), site,
+             float(p), _ptr(dz), _ptr(dy), _ptr(dgamma), _ptr(dbeta), _stream(), kernels=2)
+    return dz, dy, dgamma, dbeta
+
+
+def gelu_dropout_fwd(x, key, site, p):
+    y = torch.empty_like(x)
+    lib.call("pai_gelu_dropout_fwd", _ptr(x), x.numel(), _key(key), site, float(p), _ptr(y), _stream())
+    return y
+
+
+def gelu_dropout_bwd(x, g, key, site, p):
+    dx = torch.empty_like(x)
+    lib.call("pai_gelu_dropout_bwd", _ptr(x), _ptr(g), x.numel(), _key(key), site, float(p), _ptr(dx), _stream())
+    return dx
+
+
 # ------------------------------------------------------------------------------------------ fp32 check path
 def check_conv2d(x, w, bias=None, stride=2, pad=1, pre_act=ACT_NONE, slope=0.2, transposed=False):
     """nn.Conv2d / nn.ConvTranspose2d on fp32 NCHW (csrc/check_f32.cu): exact-arithmetic twin of the igemm layers."""
