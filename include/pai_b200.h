@@ -210,6 +210,18 @@ int pai_smallc_conv_wgrad(const void* a, int lda, int c, const float* plane0, co
  *   pai_pointwise_wgrad dw[cu][cs] += sum_r u[r, cu] * s[r, cs]                         (m % 64 == 0)
  *   pai_col2im4x4s2    out[n,2a+py,2b+px] = act(bias + sum of the 4 (tap, neighbour) partial products of
  *                      p[n,h,w,16])  -- the transposed 4x4 stride-2 conv with one output channel.
+ * Multi-plane twins for 1-4 image planes (grayscale, RGB, RGBA: the Attention U-Net's Conv2d(C, 64, 4, 2, 1) input layer
+ * and ConvTranspose2d(128, C, 4, 2, 1) output layer).  `planes` / `out` are fp32 NCHW: plane j of image n is the [h, w]
+ * image at base + (n*np + j)*plane_stride (plane_stride >= h*w; h*w for a contiguous [n, np, h, w] tensor).  np must be
+ * 1..4; the pointers must be non-null, the planes 4-byte and col 16-byte aligned.
+ *   pai_im2col4x4_planes    TAP-MAJOR columns: col[n,oy,ox, t*np+j] = plane_j[n, s*oy+dy_t, s*ox+dx_t]; the first 16*np
+ *                           columns are written (k_valid = 16*np).  Conv2d(np, C, 4, 2, 1) forward = this + a GEMM with
+ *                           w_packed[co][t*np+j] = W[co][j][t]; the data / weight gradients of ConvTranspose2d(C, np, 4, 2, 1)
+ *                           are this (on dL/dy) + a GEMM with w_packed[ci][t*np+j] = W[ci][j][t] / + pai_pointwise_wgrad.
+ *   pai_col2im4x4s2_planes  PLANE-MAJOR partial products: out_o[n,2a+py,2b+px] = act(bias[o] + sum of the 4 (tap, neighbour)
+ *                           values p[n,a+dy,b+dx, o*16+t]) for o < np; ldp >= 16*np.  The per-tap partial products come from
+ *                           pai_pointwise_gemm with w_packed[o*16+t][ci] = W[ci][o][t] (cout = 16*np).
+ * With np = 1 both compute exactly what pai_im2col4x4 (cin = 1) and pai_col2im4x4s2 compute.
  */
 int pai_im2col4x4(const float* plane0, const float* plane1, int cin, int n, int ih, int iw, int oh, int ow, int stride,
                   int flip, void* col, void* stream);
@@ -220,6 +232,10 @@ int pai_pointwise_wgrad(const void* u, long long m, int cu, int u_ld, const void
                         int splitk, void* stream);
 int pai_col2im4x4s2(const float* p, int ldp, int n, int h, int w, const float* bias, int act, float* out,
                     void* stream);
+int pai_im2col4x4_planes(const float* planes, int np, long long plane_stride, int n, int ih, int iw, int oh, int ow,
+                         int stride, int flip, void* col, void* stream);
+int pai_col2im4x4s2_planes(const float* p, int ldp, int n, int h, int w, const float* bias, int act, float* out, int np,
+                           long long plane_stride, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * The same degenerate layers as SINGLE-PASS tcgen05 kernels (csrc/thin.cu): the thin operand of the GEMM is built in
@@ -315,6 +331,15 @@ int pai_wgrad_finish(float* dw_tap_major, long long ab, float* grad, int zero_sr
  *                             negated when flip (Conv2d(1,C,k) forward; data gradient of Conv2d(C,1,k))
  *   pai_conv_wide_to_plane    out[p] = act(bias + sum_t sum_c x[p+off_t,c] * w[t][c])       (Conv2d(C,1,k) forward)
  *   pai_conv_plane_wide_wgrad dw[c][t] += sum_p wide[p,c] * plane[p+off_t]                  (k = 1 or 3)
+ *   Multi-plane twins for 1-4 image planes (the Res / Trans U-Net's Conv2d(np, 64, 3, padding=1) input and
+ *   Conv2d(64, np, 3, padding=1) + Tanh output layers): `planes` / `out` are fp32 NCHW, plane j of image n is the [h, w]
+ *   image at base + (n*np + j)*plane_stride (plane_stride >= h*w).  np must be 1..4; null pointers, a bad plane count,
+ *   stride or alignment are rejected before any CUDA call.  With np = 1 each gives the bits of its 1-plane twin.
+ *   pai_conv_planes_to_wide    out[p,c] = act(bias[c] + sum_j sum_t plane_j[p+off_t] * w[c][j][t])  (w = Conv2d weight
+ *                              [c, np, k, k]; with flip and w[c][o][t] = W[o][c][t]: data gradient of Conv2d(c, np, k))
+ *   pai_conv_wide_to_planes    out_o[p] = act(bias[o] + sum_t sum_c x[p+off_t,c] * w[o][t][c]), all np outputs from one
+ *                              read of x                                                (Conv2d(C, np, k) forward)
+ *   pai_conv_planes_wide_wgrad dw[c][j][t] += sum_p wide[p,c] * plane_j[p+off_t]          (k = 1 or 3)
  *   pai_gconv4_3x3_fprop      Conv2d(c, c, 3, padding=1, groups=c/4): w fp32 [c][9][4]
  *   pai_gconv4_3x3_wgrad      dw[co][t][j] += sum_p gy[p,co] * x[p+off_t, 4*(co/4)+j]
  */
@@ -345,6 +370,13 @@ int pai_conv_wide_to_plane(const void* x, int n, int h, int w, int c, int ldx, i
                            const float* bias, int act, float* out, void* stream);
 int pai_conv_plane_wide_wgrad(const float* plane, const void* wide, int ldw, int n, int h, int w, int c, int k, int pad,
                               int flip, float* dw, void* stream);
+int pai_conv_planes_to_wide(const float* planes, int np, long long plane_stride, int n, int h, int w, int k, int pad,
+                            int flip, const float* wt, const float* bias, int c, int act, float slope, void* out, int ldo,
+                            void* stream);
+int pai_conv_wide_to_planes(const void* x, int n, int h, int w, int c, int ldx, int k, int pad, const float* wt,
+                            const float* bias, int act, float* out, int np, long long plane_stride, void* stream);
+int pai_conv_planes_wide_wgrad(const float* planes, int np, long long plane_stride, const void* wide, int ldw, int n,
+                               int h, int w, int c, int k, int pad, int flip, float* dw, void* stream);
 int pai_gconv4_3x3_fprop(const void* x, int n, int h, int w, int c, int ldx, const float* wt, const float* bias, void* y,
                          int ldy, void* stream);
 int pai_gconv4_3x3_wgrad(const void* x, int ldx, const void* gy, int ldg, int n, int h, int w, int c, float* dw,

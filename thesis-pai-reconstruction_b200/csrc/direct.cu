@@ -3,6 +3,7 @@
 //   enc0  Conv2d(1, 64, 4, 2, 1)            models/pix2pix.py:141-147
 //   D0    Conv2d(2, 64, 4, 2, 1)+LeakyReLU  models/wrapper.py:196-206,229 (input = cat([x, y], 1))
 //   dec7  ConvTranspose2d(128, 1, 4, 2, 1)  models/pix2pix.py:186-192   (data / weight gradient)
+// plus the im2col / col2im halves of the Attention U-Net's first and last layers with 1-4 image planes.
 //   D4    Conv2d(512, 1, 4, 1, 1, no bias)  models/wrapper.py:233       (data / weight gradient)
 //
 //   pai_smallc_conv_fprop:  out[n,oy,ox,c] = act(bias[c] + sum_{t,j} plane_j[n, s*oy+dy_t, s*ox+dx_t] * W[c][t][j])
@@ -201,39 +202,44 @@ smallc_wgrad_kernel(const __nv_bfloat16* __restrict__ a, int lda, const float* _
     }
 }
 
-// im2col of 1 or 2 single-channel fp32 planes into a 64-channel bf16 NHWC tensor on the coarse grid:
+// Base pointers of up to 4 fp32 planes; plane j of image n is the [ih, iw] image at p[j] + n * img.
+struct PlaneRefs {
+    const float* p[4];
+    long long img;
+};
+__device__ __forceinline__ const float* plane_ref(const PlaneRefs& r, int j) {
+    return j == 0 ? r.p[0] : j == 1 ? r.p[1] : j == 2 ? r.p[2] : r.p[3];   // no dynamic indexing of the parameter block
+}
+
+// im2col of 1 to 4 single-channel fp32 planes into a 64-channel bf16 NHWC tensor on the coarse grid, tap-major:
 // col[n,oy,ox, t*cin + j] = plane_j[n, s*oy+dy_t, s*ox+dx_t]  (0 outside the image), rows are 64 channels wide.
-// It turns the 1-2 channel wide convolutions into plain tensor-core GEMMs (pai_pointwise_gemm / _wgrad).
+// It turns the 1-4 channel wide convolutions into plain tensor-core GEMMs (pai_pointwise_gemm / _wgrad).
 __global__ void __launch_bounds__(kDcThreads)
-im2col4x4_kernel(const float* __restrict__ p0, const float* __restrict__ p1, SmallConvGeom g,
-                 __nv_bfloat16* __restrict__ col) {
+im2col4x4_kernel(PlaneRefs pl, SmallConvGeom g, __nv_bfloat16* __restrict__ col) {
     // 2 * cin vectors of 8 channels per pixel hold data; the padding up to 64 channels is NOT written (the GEMMs that
-    // read col skip it: k_valid of pai_pointwise_gemm, discarded columns of pai_pointwise_wgrad) -- 4x / 2x less
+    // read col skip it: k_valid of pai_pointwise_gemm, discarded columns of pai_pointwise_wgrad) -- up to 4x less
     // store traffic than zero-filling the 128-byte rows
-    const unsigned nvec = 2u * (unsigned)g.cin, shift = g.cin == 2 ? 2u : 1u;
+    const unsigned nvec = 2u * (unsigned)g.cin;
     const unsigned total = (unsigned)g.n * g.oh * g.ow * nvec;
     for (unsigned idx = blockIdx.x * kDcThreads + threadIdx.x; idx < total; idx += gridDim.x * kDcThreads) {
-        const int vec = idx & (nvec - 1);
-        const unsigned pix = idx >> shift;
+        const int vec = (int)(idx % nvec);
+        const unsigned pix = idx / nvec;
         const int ox = (int)(pix % (unsigned)g.ow);
         const unsigned row = pix / (unsigned)g.ow;
         const int oy = (int)(row % (unsigned)g.oh);
         const int n = (int)(row / (unsigned)g.oh);
-        const size_t plane_off = (size_t)n * g.ih * g.iw;
+        const long long plane_off = (long long)n * pl.img;
         float v[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
             const int ch = vec * 8 + i;
-            const int t = g.cin == 2 ? ch >> 1 : ch;
-            const int j = g.cin == 2 ? ch & 1 : 0;
+            const int t = ch / g.cin;
+            const int j = ch - t * g.cin;
+            int dy, dx;
+            tap_offset(t, g.flip, &dy, &dx);
+            const int iy = oy * g.stride + dy, ix = ox * g.stride + dx;
             float x = 0.f;
-            if (t < 16) {
-                int dy, dx;
-                tap_offset(t, g.flip, &dy, &dx);
-                const int iy = oy * g.stride + dy, ix = ox * g.stride + dx;
-                if (iy >= 0 && iy < g.ih && ix >= 0 && ix < g.iw)
-                    x = __ldg((j == 0 ? p0 : p1) + plane_off + (size_t)iy * g.iw + ix);
-            }
+            if (iy >= 0 && iy < g.ih && ix >= 0 && ix < g.iw) x = __ldg(plane_ref(pl, j) + plane_off + (long long)iy * g.iw + ix);
             v[i] = x;
         }
         uint4 u;
@@ -244,32 +250,34 @@ im2col4x4_kernel(const float* __restrict__ p0, const float* __restrict__ p1, Sma
     }
 }
 
-// col2im of a transposed 4x4 stride-2 convolution with ONE output channel:
-// out[n, 2a+py, 2b+px] = act(bias + sum_{(ky,dy) in T[py]} sum_{(kx,dx) in T[px]} P[n, a+dy, b+dx, ky*4+kx])
-// P: fp32 [n, h, w, ldp] (the 16 per-tap partial products of pai_pointwise_gemm); thread <-> output pixel.
+// col2im of a transposed 4x4 stride-2 convolution with np (1..4) output channels, plane-major partial products:
+// out_o[n, 2a+py, 2b+px] = act(bias[o] + sum_{(ky,dy) in T[py]} sum_{(kx,dx) in T[px]} P[n, a+dy, b+dx, o*16 + ky*4+kx])
+// P: fp32 [n, h, w, ldp] (the 16*np per-tap partial products of pai_pointwise_gemm); thread <-> output pixel.
+// Output plane o of image n is the [2h, 2w] image at out + n*img + o*ps.
 __global__ void __launch_bounds__(kDcThreads)
 col2im4x4s2_kernel(const float* __restrict__ P, int ldp, int n, int h, int w, const float* __restrict__ bias,
-                   int act, float* __restrict__ out) {
-    const unsigned total = (unsigned)n * 4 * h * w;
+                   int act, float* __restrict__ out, int np, long long img, long long ps) {
+    const unsigned total = (unsigned)n * np * 4 * h * w;
     const int ow = 2 * w, oh = 2 * h;
     for (unsigned idx = blockIdx.x * kDcThreads + threadIdx.x; idx < total; idx += gridDim.x * kDcThreads) {
         const int x = (int)(idx % (unsigned)ow);
         const unsigned r = idx / (unsigned)ow;
         const int y = (int)(r % (unsigned)oh);
-        const int img = (int)(r / (unsigned)oh);
+        const unsigned pl = r / (unsigned)oh;
+        const int img_i = (int)(pl / (unsigned)np), o = (int)(pl % (unsigned)np);
         const int a = y >> 1, py = y & 1, b = x >> 1, px = x & 1;
         // T[0] = {(k=1,d=0),(k=3,d=-1)}, T[1] = {(k=0,d=+1),(k=2,d=0)}
         const int ky0 = py ? 0 : 1, dy0 = py ? 1 : 0, ky1 = py ? 2 : 3, dy1 = py ? 0 : -1;
         const int kx0 = px ? 0 : 1, dx0 = px ? 1 : 0, kx1 = px ? 2 : 3, dx1 = px ? 0 : -1;
-        float s = bias != nullptr ? bias[0] : 0.f;
-        const float* base = P + (size_t)img * h * w * ldp;
+        float s = bias != nullptr ? bias[o] : 0.f;
+        const float* base = P + (size_t)img_i * h * w * ldp + o * 16;
 #define PAI_TAP(ky, dy, kx, dx)                                                            \
     if (a + (dy) >= 0 && a + (dy) < h && b + (dx) >= 0 && b + (dx) < w)                    \
         s += __ldg(base + ((size_t)(a + (dy)) * w + (b + (dx))) * ldp + (ky) * 4 + (kx));
         PAI_TAP(ky0, dy0, kx0, dx0) PAI_TAP(ky0, dy0, kx1, dx1) PAI_TAP(ky1, dy1, kx0, dx0) PAI_TAP(ky1, dy1, kx1, dx1)
 #undef PAI_TAP
         if (act == PAI_ACT_TANH) s = tanhf(s);
-        out[idx] = s;
+        out[(long long)img_i * img + (long long)o * ps + (long long)y * ow + x] = s;
     }
 }
 
@@ -279,25 +287,65 @@ using namespace pai;
 
 extern "C" {
 
+static int launch_im2col4x4(const PlaneRefs& pl, int cin, int n, int ih, int iw, int oh, int ow, int stride, int flip,
+                            void* col, void* stream) {
+    SmallConvGeom g{n, ih, iw, oh, ow, stride, flip, cin, 64};
+    long long blocks = ((long long)n * oh * ow * 2 * cin + kDcThreads - 1) / kDcThreads;
+    if (blocks > 148 * 16) blocks = 148 * 16;
+    im2col4x4_kernel<<<(int)blocks, kDcThreads, 0, (cudaStream_t)stream>>>(pl, g, (__nv_bfloat16*)col);
+    PAI_CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
 int pai_im2col4x4(const float* plane0, const float* plane1, int cin, int n, int ih, int iw, int oh, int ow, int stride,
                   int flip, void* col, void* stream) {
     PAI_REQUIRE(plane0 && col && (cin == 1 || (cin == 2 && plane1)), "pai_im2col4x4: bad planes / cin=%d", cin);
     PAI_REQUIRE((long long)n * oh * ow * 8 < (1LL << 31), "pai_im2col4x4: tensor too large");
-    SmallConvGeom g{n, ih, iw, oh, ow, stride, flip, cin, 64};
-    long long blocks = ((long long)n * oh * ow * 2 * cin + kDcThreads - 1) / kDcThreads;
+    const PlaneRefs pl{{plane0, plane1, nullptr, nullptr}, (long long)ih * iw};
+    return launch_im2col4x4(pl, cin, n, ih, iw, oh, ow, stride, flip, col, stream);
+}
+
+int pai_im2col4x4_planes(const float* planes, int np, long long plane_stride, int n, int ih, int iw, int oh, int ow,
+                         int stride, int flip, void* col, void* stream) {
+    PAI_REQUIRE(planes && col, "pai_im2col4x4_planes: null pointer");
+    PAI_REQUIRE(np >= 1 && np <= 4, "pai_im2col4x4_planes: plane count %d outside 1..4", np);
+    PAI_REQUIRE(n > 0 && ih > 0 && iw > 0 && oh > 0 && ow > 0 && plane_stride >= (long long)ih * iw,
+                "pai_im2col4x4_planes: bad size / plane stride %lld", plane_stride);
+    PAI_REQUIRE((reinterpret_cast<uintptr_t>(planes) & 3) == 0 && (reinterpret_cast<uintptr_t>(col) & 15) == 0,
+                "pai_im2col4x4_planes: alignment");
+    PAI_REQUIRE((long long)n * oh * ow * 8 < (1LL << 31), "pai_im2col4x4_planes: tensor too large");
+    PlaneRefs pl{{planes, planes, planes, planes}, np * plane_stride};
+    for (int j = 1; j < np; ++j) pl.p[j] = planes + j * plane_stride;
+    return launch_im2col4x4(pl, np, n, ih, iw, oh, ow, stride, flip, col, stream);
+}
+
+static void col2im4x4s2_launch(const float* p, int ldp, int n, int h, int w, const float* bias, int act, float* out,
+                               int np, long long img, long long ps, void* stream) {
+    long long blocks = ((long long)n * np * 4 * h * w + kDcThreads - 1) / kDcThreads;
     if (blocks > 148 * 16) blocks = 148 * 16;
-    im2col4x4_kernel<<<(int)blocks, kDcThreads, 0, (cudaStream_t)stream>>>(plane0, plane1, g, (__nv_bfloat16*)col);
-    PAI_CUDA_OK(cudaGetLastError());
-    return 0;
+    col2im4x4s2_kernel<<<(int)blocks, kDcThreads, 0, (cudaStream_t)stream>>>(p, ldp, n, h, w, bias, act, out, np, img, ps);
 }
 
 int pai_col2im4x4s2(const float* p, int ldp, int n, int h, int w, const float* bias, int act, float* out,
                     void* stream) {
     PAI_REQUIRE(p && out && ldp >= 16, "pai_col2im4x4s2: null pointer / ldp < 16");
     PAI_REQUIRE((long long)n * 4 * h * w < (1LL << 31), "pai_col2im4x4s2: tensor too large");
-    long long blocks = ((long long)n * 4 * h * w + kDcThreads - 1) / kDcThreads;
-    if (blocks > 148 * 16) blocks = 148 * 16;
-    col2im4x4s2_kernel<<<(int)blocks, kDcThreads, 0, (cudaStream_t)stream>>>(p, ldp, n, h, w, bias, act, out);
+    const long long hw4 = 4LL * h * w;
+    col2im4x4s2_launch(p, ldp, n, h, w, bias, act, out, 1, hw4, hw4, stream);
+    PAI_CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
+int pai_col2im4x4s2_planes(const float* p, int ldp, int n, int h, int w, const float* bias, int act, float* out, int np,
+                           long long plane_stride, void* stream) {
+    PAI_REQUIRE(p && out, "pai_col2im4x4s2_planes: null pointer");
+    PAI_REQUIRE(np >= 1 && np <= 4, "pai_col2im4x4s2_planes: plane count %d outside 1..4", np);
+    PAI_REQUIRE(n > 0 && h > 0 && w > 0 && ldp >= 16 * np && plane_stride >= 4LL * h * w,
+                "pai_col2im4x4s2_planes: bad size, ldp %d < 16 * planes or plane stride %lld", ldp, plane_stride);
+    PAI_REQUIRE((reinterpret_cast<uintptr_t>(p) & 3) == 0 && (reinterpret_cast<uintptr_t>(out) & 3) == 0,
+                "pai_col2im4x4s2_planes: alignment");
+    PAI_REQUIRE((long long)n * np * 4 * h * w < (1LL << 31), "pai_col2im4x4s2_planes: tensor too large");
+    col2im4x4s2_launch(p, ldp, n, h, w, bias, act, out, np, np * plane_stride, plane_stride, stream);
     PAI_CUDA_OK(cudaGetLastError());
     return 0;
 }

@@ -7,7 +7,7 @@
 //   nn.MaxPool2d(2) / nn.Upsample(scale_factor=2)         models/res_unet.py:196,228; models/trans_unet.py
 //   residual add (+ReLU)                                   models/res_unet.py:90,129-130,170-171
 //   x * attention                                          models/attention_unet.py:96
-//   Conv2d(1, 64, 3, padding=1) / Conv2d(64, 1, 3, padding=1) (+Tanh)   models/res_unet.py:263,312-320
+//   Conv2d(C, 64, 3, padding=1) / Conv2d(64, C, 3, padding=1) (+Tanh), C = 1..4   models/res_unet.py:263,312-320
 //   Conv2d(C/2, 1, 1) of the attention gate                models/attention_unet.py:85-89
 //   Conv2d(128, 128, 3, padding=1, groups=32) (ResNeXt)    models/res_unet.py:150-156
 #include "pai_common.cuh"
@@ -254,18 +254,21 @@ scale_rows_bwd_kernel(const __nv_bfloat16* __restrict__ x, int ldx, const float*
 }
 
 // ---------------------------------------------------------------------------------------------
-// 1-channel <-> C-channel k x k convolutions (stride 1, zero padding `pad`), taps t = ky*k + kx at offset
-// (ky - pad, kx - pad), negated when `flip`.
-//   plane_to_wide:  out[p, c] = act(bias[c] + sum_t plane[p + off_t] * w[c][t])
-//   wide_to_plane:  out[p]    = act(bias + sum_t sum_c x[p + off_t, c] * w[t][c])
-//   plane_wide_wgrad: dw[c][t] += sum_p wide[p, c] * plane[p + off_t]
+// P-plane (1 <= P <= 4) <-> C-channel k x k convolutions (stride 1, zero padding `pad`), taps t = ky*k + kx at offset
+// (ky - pad, kx - pad), negated when `flip`.  Plane j of image b is the fp32 [h, w] image at base + b*img + j*ps
+// (NCHW [n, P, h, w]: ps = h*w, img = P*h*w; a 1-plane [n, h, w] tensor is img = h*w).
+//   plane_to_wide:  out[p, c]  = act(bias[c] + sum_j sum_t plane_j[p + off_t] * w[c][j][t])
+//   wide_to_plane:  out_o[p]   = act(bias[o] + sum_t sum_c x[p + off_t, c] * w[o][t][c])      (o < P)
+//   plane_wide_wgrad: dw[c][j][t] += sum_p wide[p, c] * plane_j[p + off_t]
+// With P = 1 every kernel issues the FMAs of the original 1-plane kernels in the same order, so the 1-plane entry
+// points (which call these kernels) give the same bits as before.
 __global__ void __launch_bounds__(kLyThreads)
-plane_to_wide_kernel(const float* __restrict__ plane, int n, int h, int w, int k, int pad, int flip,
-                     const float* __restrict__ wt /* [c][k*k] */, const float* __restrict__ bias, int c, int act,
-                     float slope, __nv_bfloat16* __restrict__ out, int ldo) {
-    extern __shared__ float wsm[];   // [k*k][c]
-    const int taps = k * k;
-    for (int i = threadIdx.x; i < c * taps; i += kLyThreads) wsm[(i % taps) * c + i / taps] = wt[i];
+plane_to_wide_kernel(const float* __restrict__ planes, long long img, long long ps, int np, int n, int h, int w, int k,
+                     int pad, int flip, const float* __restrict__ wt /* [c][np][k*k] */, const float* __restrict__ bias,
+                     int c, int act, float slope, __nv_bfloat16* __restrict__ out, int ldo) {
+    extern __shared__ float wsm[];   // [np*k*k][c]
+    const int taps = k * k, rows = np * taps;
+    for (int i = threadIdx.x; i < c * rows; i += kLyThreads) wsm[(i % rows) * c + i / rows] = wt[i];
     __syncthreads();
     const int cv = c >> 3;
     const long long total = (long long)n * h * w * cv;
@@ -279,15 +282,18 @@ plane_to_wide_kernel(const float* __restrict__ plane, int n, int h, int w, int k
         V8 acc;
 #pragma unroll
         for (int q = 0; q < 8; ++q) acc.v[q] = bias != nullptr ? bias[vec * 8 + q] : 0.f;
-        for (int t = 0; t < taps; ++t) {
-            int dy = t / k - pad, dx = t % k - pad;
-            if (flip) dy = -dy, dx = -dx;
-            const int yy = y0 + dy, xx = x0 + dx;
-            if (yy < 0 || yy >= h || xx < 0 || xx >= w) continue;
-            const float v = __ldg(plane + ((long long)b * h + yy) * w + xx);
-            const float* wr = wsm + t * c + vec * 8;
+        for (int j = 0; j < np; ++j) {
+            const float* src = planes + (long long)b * img + (long long)j * ps;
+            for (int t = 0; t < taps; ++t) {
+                int dy = t / k - pad, dx = t % k - pad;
+                if (flip) dy = -dy, dx = -dx;
+                const int yy = y0 + dy, xx = x0 + dx;
+                if (yy < 0 || yy >= h || xx < 0 || xx >= w) continue;
+                const float v = __ldg(src + (long long)yy * w + xx);
+                const float* wr = wsm + (j * taps + t) * c + vec * 8;
 #pragma unroll
-            for (int q = 0; q < 8; ++q) acc.v[q] = fmaf(v, wr[q], acc.v[q]);
+                for (int q = 0; q < 8; ++q) acc.v[q] = fmaf(v, wr[q], acc.v[q]);
+            }
         }
 #pragma unroll
         for (int q = 0; q < 8; ++q) acc.v[q] = act_apply(acc.v[q], act, slope);
@@ -295,58 +301,78 @@ plane_to_wide_kernel(const float* __restrict__ plane, int n, int h, int w, int k
     }
 }
 
-// 8 lanes per pixel (channel vectors strided by 8), shuffle reduce
+// 8 lanes per pixel (channel vectors strided by 8), shuffle reduce; all P output planes from one read of x
+template <int P>
 __global__ void __launch_bounds__(kLyThreads)
 wide_to_plane_kernel(const __nv_bfloat16* __restrict__ x, int n, int h, int w, int c, int ldx, int k, int pad,
-                     const float* __restrict__ wt /* [k*k][c] */, const float* __restrict__ bias, int act,
-                     float* __restrict__ out) {
-    const int cv = c >> 3, sub = threadIdx.x & 7;
+                     const float* __restrict__ wt /* [P][k*k][c] */, const float* __restrict__ bias, int act,
+                     float* __restrict__ out, long long img, long long ps) {
+    const int cv = c >> 3, sub = threadIdx.x & 7, taps = k * k;
     const long long total = (long long)n * h * w;
     const long long g0 = ((long long)blockIdx.x * kLyThreads + threadIdx.x) >> 3;
     const long long ng = ((long long)gridDim.x * kLyThreads) >> 3;
     const long long rounds = (total + ng - 1) / ng;
     for (long long it = 0; it < rounds; ++it) {
         const long long p = g0 + it * ng;
-        float acc = 0.f;
+        float acc[P];
+#pragma unroll
+        for (int o = 0; o < P; ++o) acc[o] = 0.f;
+        int x0 = 0, y0 = 0, b = 0;
         if (p < total) {
-            const int x0 = (int)(p % w);
-            const int y0 = (int)((p / w) % h);
-            const int b = (int)(p / ((long long)w * h));
-            for (int t = 0; t < k * k; ++t) {
+            x0 = (int)(p % w);
+            y0 = (int)((p / w) % h);
+            b = (int)(p / ((long long)w * h));
+            for (int t = 0; t < taps; ++t) {
                 const int yy = y0 + t / k - pad, xx = x0 + t % k - pad;
                 if (yy < 0 || yy >= h || xx < 0 || xx >= w) continue;
                 const __nv_bfloat16* src = x + (((long long)b * h + yy) * w + xx) * ldx;
                 for (int vec = sub; vec < cv; vec += 8) {
                     const V8 v = ld8(src + vec * 8);
-                    const float* wr = wt + (long long)t * c + vec * 8;
 #pragma unroll
-                    for (int q = 0; q < 8; ++q) acc = fmaf(v.v[q], __ldg(wr + q), acc);
+                    for (int o = 0; o < P; ++o) {
+                        const float* wr = wt + ((long long)o * taps + t) * c + vec * 8;
+#pragma unroll
+                        for (int q = 0; q < 8; ++q) acc[o] = fmaf(v.v[q], __ldg(wr + q), acc[o]);
+                    }
                 }
             }
         }
-        acc += __shfl_xor_sync(0xffffffffu, acc, 1);
-        acc += __shfl_xor_sync(0xffffffffu, acc, 2);
-        acc += __shfl_xor_sync(0xffffffffu, acc, 4);
-        if (p < total && sub == 0) out[p] = act_apply(acc + (bias != nullptr ? bias[0] : 0.f), act, 0.f);
+#pragma unroll
+        for (int o = 0; o < P; ++o) {
+            acc[o] += __shfl_xor_sync(0xffffffffu, acc[o], 1);
+            acc[o] += __shfl_xor_sync(0xffffffffu, acc[o], 2);
+            acc[o] += __shfl_xor_sync(0xffffffffu, acc[o], 4);
+        }
+        if (p < total && sub == 0) {
+            float* dst = out + (long long)b * img + (long long)y0 * w + x0;
+#pragma unroll
+            for (int o = 0; o < P; ++o) dst[(long long)o * ps] = act_apply(acc[o] + (bias != nullptr ? bias[o] : 0.f), act, 0.f);
+        }
     }
 }
 
-// thread <-> (pixel, 8 channels); per-thread partial sums for all taps (<= 9), block reduce, atomics
+// thread <-> (pixel, 8 channels); per-thread partial sums for all taps (<= 9) of ONE plane, block reduce, atomics.
+// The planes are spread over the grid (block = pixel block * np + plane), so a thread never holds more than
+// TAPS x 8 accumulators whatever np is; the np blocks of a pixel block run side by side and share the wide reads in L2.
 template <int TAPS>
 __global__ void __launch_bounds__(kLyThreads)
-plane_wide_wgrad_kernel(const float* __restrict__ plane, const __nv_bfloat16* __restrict__ wide, int ldw, int n, int h,
-                        int w, int c, int k, int pad, int flip, float* __restrict__ dw /* [c][TAPS] */) {
+plane_wide_wgrad_kernel(const float* __restrict__ planes, long long img, long long ps, int np,
+                        const __nv_bfloat16* __restrict__ wide, int ldw, int n, int h, int w, int c, int k, int pad,
+                        int flip, float* __restrict__ dw /* [c][np][TAPS] */) {
     __shared__ float red[kLyThreads * 8];
     const int cv = c >> 3;
     const int vec = threadIdx.x % cv;
     const int ppb = kLyThreads / cv;
+    const int j = (int)(blockIdx.x % (unsigned)np);
+    const long long blk = blockIdx.x / (unsigned)np, nblk = gridDim.x / (unsigned)np;
+    const float* src = planes + (long long)j * ps;
     float acc[TAPS][8];
 #pragma unroll
     for (int t = 0; t < TAPS; ++t)
 #pragma unroll
         for (int q = 0; q < 8; ++q) acc[t][q] = 0.f;
     const long long total = (long long)n * h * w;
-    for (long long p = (long long)blockIdx.x * ppb + threadIdx.x / cv; p < total; p += (long long)gridDim.x * ppb) {
+    for (long long p = blk * ppb + threadIdx.x / cv; p < total; p += nblk * ppb) {
         const int x0 = (int)(p % w);
         const int y0 = (int)((p / w) % h);
         const int b = (int)(p / ((long long)w * h));
@@ -356,7 +382,7 @@ plane_wide_wgrad_kernel(const float* __restrict__ plane, const __nv_bfloat16* __
             int dy = t / k - pad, dx = t % k - pad;
             if (flip) dy = -dy, dx = -dx;
             const int yy = y0 + dy, xx = x0 + dx;
-            const float s = (yy >= 0 && yy < h && xx >= 0 && xx < w) ? __ldg(plane + ((long long)b * h + yy) * w + xx) : 0.f;
+            const float s = (yy >= 0 && yy < h && xx >= 0 && xx < w) ? __ldg(src + (long long)b * img + (long long)yy * w + xx) : 0.f;
 #pragma unroll
             for (int q = 0; q < 8; ++q) acc[t][q] = fmaf(v.v[q], s, acc[t][q]);
         }
@@ -371,7 +397,7 @@ plane_wide_wgrad_kernel(const float* __restrict__ plane, const __nv_bfloat16* __
             const int vv = i >> 3, q = i & 7;
             float s = 0.f;
             for (int r = vv; r < kLyThreads; r += cv) s += red[r * 8 + q];
-            atomicAdd(dw + (long long)i * TAPS + t, s);
+            atomicAdd(dw + ((long long)i * np + j) * TAPS + t, s);
         }
     }
 }
@@ -584,40 +610,101 @@ int pai_scale_rows_bwd(const void* x, int ldx, const float* s, const void* g, in
     PAI_CUDA_OK(cudaGetLastError());
     return 0;
 }
+static bool planes_ok(int np, long long ps, int h, int w, const void* p) {
+    return np >= 1 && np <= 4 && ps >= (long long)h * w && (reinterpret_cast<uintptr_t>(p) & 3) == 0;
+}
+static int launch_plane_to_wide(const char* who, const float* planes, long long img, long long ps, int np, int n, int h,
+                                int w, int k, int pad, int flip, const float* wt, const float* bias, int c, int act,
+                                float slope, void* out, int ldo, void* stream) {
+    PAI_REQUIRE(v8_ok(c, out, ldo) && c * np * k * k * 4 <= 48 * 1024, "%s: bad channels / alignment", who);
+    plane_to_wide_kernel<<<ly_grid((long long)n * h * w * (c / 8)), kLyThreads, c * np * k * k * sizeof(float),
+                           (cudaStream_t)stream>>>(planes, img, ps, np, n, h, w, k, pad, flip, wt, bias, c, act, slope,
+                                                   (bf16*)out, ldo);
+    PAI_CUDA_OK(cudaGetLastError());
+    return 0;
+}
+static int launch_wide_to_plane(const void* x, int n, int h, int w, int c, int ldx, int k, int pad, const float* wt,
+                                const float* bias, int act, float* out, int np, long long img, long long ps, void* stream) {
+    const int grid = ly_grid((long long)n * h * w * 8);
+    cudaStream_t st = (cudaStream_t)stream;
+    switch (np) {
+        case 1: wide_to_plane_kernel<1><<<grid, kLyThreads, 0, st>>>((const bf16*)x, n, h, w, c, ldx, k, pad, wt, bias, act, out, img, ps); break;
+        case 2: wide_to_plane_kernel<2><<<grid, kLyThreads, 0, st>>>((const bf16*)x, n, h, w, c, ldx, k, pad, wt, bias, act, out, img, ps); break;
+        case 3: wide_to_plane_kernel<3><<<grid, kLyThreads, 0, st>>>((const bf16*)x, n, h, w, c, ldx, k, pad, wt, bias, act, out, img, ps); break;
+        default: wide_to_plane_kernel<4><<<grid, kLyThreads, 0, st>>>((const bf16*)x, n, h, w, c, ldx, k, pad, wt, bias, act, out, img, ps); break;
+    }
+    PAI_CUDA_OK(cudaGetLastError());
+    return 0;
+}
+static int launch_plane_wide_wgrad(const char* who, const float* planes, long long img, long long ps, int np,
+                                   const void* wide, int ldw, int n, int h, int w, int c, int k, int pad, int flip,
+                                   float* dw, void* stream) {
+    PAI_REQUIRE(k == 1 || k == 3, "%s: k must be 1 or 3 (got %d)", who, k);
+    PAI_REQUIRE(v8_ok(c, wide, ldw) && cv_divides_block(c), "%s: bad channels / alignment (c=%d)", who, c);
+    const long long ppb = kLyThreads / (c / 8);
+    long long blocks = ((long long)n * h * w + ppb - 1) / ppb;
+    if (blocks > 148 * 4) blocks = 148 * 4;
+    blocks *= np;
+    if (k == 1)
+        plane_wide_wgrad_kernel<1><<<(int)blocks, kLyThreads, 0, (cudaStream_t)stream>>>(planes, img, ps, np, (const bf16*)wide,
+                                                                                       ldw, n, h, w, c, k, pad, flip, dw);
+    else
+        plane_wide_wgrad_kernel<9><<<(int)blocks, kLyThreads, 0, (cudaStream_t)stream>>>(planes, img, ps, np, (const bf16*)wide,
+                                                                                       ldw, n, h, w, c, k, pad, flip, dw);
+    PAI_CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
 int pai_conv_plane_to_wide(const float* plane, int n, int h, int w, int k, int pad, int flip, const float* wt,
                            const float* bias, int c, int act, float slope, void* out, int ldo, void* stream) {
     PAI_REQUIRE(plane && wt && out && n > 0 && k >= 1 && k <= 4, "pai_conv_plane_to_wide: null pointer or k=%d", k);
-    PAI_REQUIRE(v8_ok(c, out, ldo) && c * k * k * 4 <= 48 * 1024, "pai_conv_plane_to_wide: bad channels / alignment");
-    plane_to_wide_kernel<<<ly_grid((long long)n * h * w * (c / 8)), kLyThreads, c * k * k * sizeof(float),
-                           (cudaStream_t)stream>>>(plane, n, h, w, k, pad, flip, wt, bias, c, act, slope, (bf16*)out, ldo);
-    PAI_CUDA_OK(cudaGetLastError());
-    return 0;
+    const long long hw = (long long)h * w;
+    return launch_plane_to_wide("pai_conv_plane_to_wide", plane, hw, hw, 1, n, h, w, k, pad, flip, wt, bias, c, act, slope,
+                                out, ldo, stream);
+}
+int pai_conv_planes_to_wide(const float* planes, int np, long long plane_stride, int n, int h, int w, int k, int pad,
+                            int flip, const float* wt, const float* bias, int c, int act, float slope, void* out, int ldo,
+                            void* stream) {
+    PAI_REQUIRE(planes && wt && out, "pai_conv_planes_to_wide: null pointer");
+    PAI_REQUIRE(np >= 1 && np <= 4, "pai_conv_planes_to_wide: plane count %d outside 1..4", np);
+    PAI_REQUIRE(n > 0 && h > 0 && w > 0 && k >= 1 && k <= 4, "pai_conv_planes_to_wide: bad size or k=%d", k);
+    PAI_REQUIRE(planes_ok(np, plane_stride, h, w, planes), "pai_conv_planes_to_wide: plane stride %lld / alignment",
+                plane_stride);
+    return launch_plane_to_wide("pai_conv_planes_to_wide", planes, np * plane_stride, plane_stride, np, n, h, w, k, pad, flip,
+                                wt, bias, c, act, slope, out, ldo, stream);
 }
 int pai_conv_wide_to_plane(const void* x, int n, int h, int w, int c, int ldx, int k, int pad, const float* wt,
                            const float* bias, int act, float* out, void* stream) {
     PAI_REQUIRE(x && wt && out && n > 0 && k >= 1 && k <= 4, "pai_conv_wide_to_plane: null pointer or k=%d", k);
     PAI_REQUIRE(v8_ok(c, x, ldx), "pai_conv_wide_to_plane: bad channels / alignment");
-    wide_to_plane_kernel<<<ly_grid((long long)n * h * w * 8), kLyThreads, 0, (cudaStream_t)stream>>>(
-        (const bf16*)x, n, h, w, c, ldx, k, pad, wt, bias, act, out);
-    PAI_CUDA_OK(cudaGetLastError());
-    return 0;
+    const long long hw = (long long)h * w;
+    return launch_wide_to_plane(x, n, h, w, c, ldx, k, pad, wt, bias, act, out, 1, hw, hw, stream);
+}
+int pai_conv_wide_to_planes(const void* x, int n, int h, int w, int c, int ldx, int k, int pad, const float* wt,
+                            const float* bias, int act, float* out, int np, long long plane_stride, void* stream) {
+    PAI_REQUIRE(x && wt && out, "pai_conv_wide_to_planes: null pointer");
+    PAI_REQUIRE(np >= 1 && np <= 4, "pai_conv_wide_to_planes: plane count %d outside 1..4", np);
+    PAI_REQUIRE(n > 0 && h > 0 && w > 0 && k >= 1 && k <= 4, "pai_conv_wide_to_planes: bad size or k=%d", k);
+    PAI_REQUIRE(v8_ok(c, x, ldx) && planes_ok(np, plane_stride, h, w, out),
+                "pai_conv_wide_to_planes: bad channels / plane stride / alignment");
+    return launch_wide_to_plane(x, n, h, w, c, ldx, k, pad, wt, bias, act, out, np, np * plane_stride, plane_stride, stream);
 }
 int pai_conv_plane_wide_wgrad(const float* plane, const void* wide, int ldw, int n, int h, int w, int c, int k, int pad,
                               int flip, float* dw, void* stream) {
     PAI_REQUIRE(plane && wide && dw && n > 0, "pai_conv_plane_wide_wgrad: null pointer");
-    PAI_REQUIRE(k == 1 || k == 3, "pai_conv_plane_wide_wgrad: k must be 1 or 3 (got %d)", k);
-    PAI_REQUIRE(v8_ok(c, wide, ldw) && cv_divides_block(c), "pai_conv_plane_wide_wgrad: bad channels / alignment (c=%d)", c);
-    const long long ppb = kLyThreads / (c / 8);
-    long long blocks = ((long long)n * h * w + ppb - 1) / ppb;
-    if (blocks > 148 * 4) blocks = 148 * 4;
-    if (k == 1)
-        plane_wide_wgrad_kernel<1><<<(int)blocks, kLyThreads, 0, (cudaStream_t)stream>>>(plane, (const bf16*)wide, ldw, n, h,
-                                                                                       w, c, k, pad, flip, dw);
-    else
-        plane_wide_wgrad_kernel<9><<<(int)blocks, kLyThreads, 0, (cudaStream_t)stream>>>(plane, (const bf16*)wide, ldw, n, h,
-                                                                                       w, c, k, pad, flip, dw);
-    PAI_CUDA_OK(cudaGetLastError());
-    return 0;
+    const long long hw = (long long)h * w;
+    return launch_plane_wide_wgrad("pai_conv_plane_wide_wgrad", plane, hw, hw, 1, wide, ldw, n, h, w, c, k, pad, flip, dw,
+                                   stream);
+}
+int pai_conv_planes_wide_wgrad(const float* planes, int np, long long plane_stride, const void* wide, int ldw, int n,
+                               int h, int w, int c, int k, int pad, int flip, float* dw, void* stream) {
+    PAI_REQUIRE(planes && wide && dw, "pai_conv_planes_wide_wgrad: null pointer");
+    PAI_REQUIRE(np >= 1 && np <= 4, "pai_conv_planes_wide_wgrad: plane count %d outside 1..4", np);
+    PAI_REQUIRE(n > 0 && h > 0 && w > 0, "pai_conv_planes_wide_wgrad: empty input");
+    PAI_REQUIRE(planes_ok(np, plane_stride, h, w, planes), "pai_conv_planes_wide_wgrad: plane stride %lld / alignment",
+                plane_stride);
+    return launch_plane_wide_wgrad("pai_conv_planes_wide_wgrad", planes, np * plane_stride, plane_stride, np, wide, ldw, n,
+                                   h, w, c, k, pad, flip, dw, stream);
 }
 int pai_gconv4_3x3_fprop(const void* x, int n, int h, int w, int c, int ldx, const float* wt, const float* bias, void* y,
                          int ldy, void* stream) {

@@ -74,7 +74,7 @@ class AttentionBlock(nn.Module):
 
 
 class AttentionUnet(nn.Module):
-    """``[N, 1, H, W] -> [N, 1, H, W]`` in (-1, 1)."""
+    """``[N, in_channels, H, W] -> [N, out_channels, H, W]`` in (-1, 1), 1 to 4 channels each."""
 
     def __init__(self, in_channels: int = 3, out_channels: int = 3,
                  channel_mults: Sequence[int] = (1, 2, 4, 8, 8, 8, 8, 8), dropout: float = 0.5):
@@ -121,9 +121,14 @@ class AttentionUnet(nn.Module):
         depth = len(self.encoders)
         if hh % (1 << depth) or ww % (1 << depth):
             raise RuntimeError(f"pai_b200: input {hh}x{ww} must be divisible by 2^{depth}")
-        h = L.to_plane(x)
-        feats = []
-        for enc in self.encoders:
+        cin, cout = self.encoders[0].in_channels, self.decoders[-1].out_channels
+        L.check_image_channels(cin, cout)
+        if cin == 1:
+            h = self._encode(self.encoders[0], L.to_plane(x))
+        else:
+            h = L.conv4x4s2_in_planes(L.to_planes(x, cin), self.encoders[0])
+        feats = [h]
+        for enc in self.encoders[1:]:
             h = self._encode(enc, h)
             feats.append(h)
         feats.pop()
@@ -132,6 +137,8 @@ class AttentionUnet(nn.Module):
             if j != 0:
                 s = self.attention_blocks[j - 1](feats.pop(), h)
                 h = torch.cat([h, s], dim=-1)
-            if j == last:
-                return L.convT4x4s2_out_tanh(h, dec).view(n, 1, hh, ww)      # bare ConvTranspose2d: no ReLU before it
+            if j == last:                                                     # bare ConvTranspose2d: no ReLU before it
+                if cout == 1:
+                    return L.convT4x4s2_out_tanh(h, dec).view(n, 1, hh, ww)
+                return L.convT4x4s2_out_planes_tanh(h, dec)
             h = self._decode(dec, h)

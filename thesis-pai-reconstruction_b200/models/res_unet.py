@@ -211,7 +211,8 @@ class DecoderBlock(nn.Module):
 
 
 class ResUnet(nn.Module):
-    """``[N, 1, H, W] -> [N, 1, H, W]`` in (-1, 1); H and W divisible by 2^len(channel_mults)."""
+    """``[N, in_channels, H, W] -> [N, out_channels, H, W]`` in (-1, 1), 1 to 4 channels each (grayscale, RGB, RGBA);
+    H and W divisible by 2^len(channel_mults)."""
 
     def __init__(self, in_channels: int = 3, out_channels: int = 3, res_type: ResType = "18",
                  channel_mults: Sequence[int] = (1, 2, 4, 8, 8, 8, 8, 8), dropout: float = 0.5):
@@ -243,7 +244,12 @@ class ResUnet(nn.Module):
         depth = len(self.encoders)
         if hh % (1 << depth) or ww % (1 << depth):
             raise RuntimeError(f"pai_b200: input {hh}x{ww} must be divisible by 2^{depth}")
-        h = L.conv_in(L.to_plane(x), self.in_conv)
+        cin, cout = self.in_conv.in_channels, self.out[0].out_channels
+        L.check_image_channels(cin, cout)
+        if cin == 1:
+            h = L.conv_in(L.to_plane(x), self.in_conv)
+        else:
+            h = L.conv_in_planes(L.to_planes(x, cin), self.in_conv)
         skips = []
         for enc in self.encoders:
             h = enc(h)
@@ -253,5 +259,7 @@ class ResUnet(nn.Module):
             if j != 0:
                 h = torch.cat([h, skips.pop()], dim=-1)      # NHWC: channel concat on the last axis
             h = dec(h)
-        y = L.conv_out(h, self.out[0], L.ACT_TANH)
-        return y.view(n, 1, hh, ww)
+        if cout == 1:
+            y = L.conv_out(h, self.out[0], L.ACT_TANH)
+            return y.view(n, 1, hh, ww)
+        return L.conv_out_planes(h, self.out[0], L.ACT_TANH)

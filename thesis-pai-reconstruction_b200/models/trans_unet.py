@@ -170,7 +170,7 @@ class VisionTransformer(nn.Module):
 
 
 class TransUnet(nn.Module):
-    """``[N, 1, 256, 256] -> [N, 1, 256, 256]`` in (-1, 1)."""
+    """``[N, in_channels, 256, 256] -> [N, out_channels, 256, 256]`` in (-1, 1), 1 to 4 channels each."""
 
     def __init__(self, in_channels: int = 3, out_channels: int = 3, image_size: int = 256,
                  channel_mults: Sequence[int] = (1, 2, 4, 8), patch_size: int = 16, num_heads: int = 8,
@@ -199,7 +199,12 @@ class TransUnet(nn.Module):
 
     def _forward(self, x):
         n, _, hh, ww = x.shape
-        h = L.conv_in(L.to_plane(x), self.in_conv)
+        cin, cout = self.in_conv.in_channels, self.out[0].out_channels
+        L.check_image_channels(cin, cout)
+        if cin == 1:
+            h = L.conv_in(L.to_plane(x), self.in_conv)
+        else:
+            h = L.conv_in_planes(L.to_planes(x, cin), self.in_conv)
         skips = []
         for enc in self.encoders:
             h = enc(h)
@@ -210,4 +215,6 @@ class TransUnet(nn.Module):
             if j != 0:
                 h = torch.cat([h, skips.pop()], dim=-1)
             h = dec(h)
-        return L.conv_out(h, self.out[0], L.ACT_TANH).view(n, 1, hh, ww)
+        if cout == 1:
+            return L.conv_out(h, self.out[0], L.ACT_TANH).view(n, 1, hh, ww)
+        return L.conv_out_planes(h, self.out[0], L.ACT_TANH)

@@ -137,7 +137,7 @@ def _pad_cols(t, cols=64):
     return out
 
 
-def _thin_in_pack(w):    # Conv2d weight [C, cin<=2, 4, 4] -> bf16 [C, 64]: column = tap*cin + j (im2col order)
+def _thin_in_pack(w):    # Conv2d weight [C, cin<=4, 4, 4] -> bf16 [C, 64]: column = tap*cin + j (im2col order)
     return _packs.get("thin_in", w, lambda t: _pad_cols(t.permute(0, 2, 3, 1).reshape(t.shape[0], -1)))
 
 
@@ -147,6 +147,14 @@ def _thin_out_fprop_pack(w):   # ConvT weight [Cin, 1, 4, 4] -> bf16 [16, Cin]: 
 
 def _thin_out_dgrad_pack(w):   # ConvT weight [Cin, 1, 4, 4] -> bf16 [Cin, 64]: column = tap
     return _packs.get("thin_out_d", w, lambda t: _pad_cols(t[:, 0].reshape(t.shape[0], 16)))
+
+
+def _planes_out_fprop_pack(w):   # ConvT weight [Cin, np, 4, 4] -> bf16 [16*np, Cin]: row = o*16 + tap (plane-major)
+    return _packs.get("planes_out_f", w, lambda t: t.reshape(t.shape[0], -1).t().contiguous().bfloat16())
+
+
+def _planes_out_dgrad_pack(w):   # ConvT weight [Cin, np, 4, 4] -> bf16 [Cin, 64]: column = tap*np + j (im2col order)
+    return _packs.get("planes_out_d", w, lambda t: _pad_cols(t.permute(0, 2, 3, 1).reshape(t.shape[0], -1)))
 
 
 def _aux_pack(tag: str, p: torch.Tensor, fn):

@@ -2,7 +2,8 @@
 (reference: models/res_unet.py, models/attention_unet.py, models/trans_unet.py).
 
 Activations travel between nodes as NHWC bf16 tensors ``[N, H, W, C]``; 1-channel tensors (network input
-and output, attention logits) are fp32 planes ``[N, H, W]``.  Parameters are the fp32 tensors of the
+and output, attention logits) are fp32 planes ``[N, H, W]``, and 2-4 channel network inputs / outputs are fp32 NCHW
+plane stacks ``[N, C, H, W]``.  Parameters are the fp32 tensors of the
 drop-in ``nn.Module`` tree in the reference's layouts.  Every node's forward AND backward is a kernel of
 libpai_b200.so; there is no PyTorch-op implementation behind them.
 """
@@ -345,6 +346,137 @@ class _ConvT4x4s2Out(torch.autograd.Function):
         return gx, gw, gb
 
 
+# ------------------------------------------------------------------------------------------ 1-4 image planes
+# Multi-channel images (RGB, RGBA, ...) enter and leave the networks as fp32 NCHW plane stacks [N, C, H, W] (what the
+# model receives and returns, no permute).  C = 1 keeps the 1-plane nodes above; C = 2..4 run the multi-plane kernels.
+MAX_PLANES = 4
+
+
+def _check_planes(c: int, what: str):
+    if not 1 <= c <= MAX_PLANES:
+        raise RuntimeError(f"pai_b200: {what}={c}: the B200 path takes 1 to {MAX_PLANES} image channels "
+                           f"(grayscale, RGB, RGBA); no fallback exists")
+
+
+def check_image_channels(in_channels: int, out_channels: int):
+    """Raises before any launch when a network's image channel counts are outside 1..4."""
+    _check_planes(in_channels, "in_channels")
+    _check_planes(out_channels, "out_channels")
+
+
+class _PlanesToWide(torch.autograd.Function):
+    """nn.Conv2d(C, c, k, padding=k//2) on fp32 planes ``[N, C, H, W]`` (the network input: no data gradient)."""
+
+    @staticmethod
+    def forward(ctx, planes, weight, bias, act):
+        c, np_, k = weight.shape[0], weight.shape[1], weight.shape[2]
+        y = ops.conv_planes_to_wide(planes, weight.detach().reshape(c, np_ * k * k), None if bias is None else bias.detach(),
+                                    k, k // 2, act)
+        ctx.save_for_backward(planes, y)
+        ctx.k, ctx.act, ctx.has_bias = k, act, bias is not None
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        planes, y = ctx.saved_tensors
+        gy = gy.contiguous()
+        if ctx.act != ACT_NONE:
+            g2 = torch.empty_like(gy)
+            ops.act_bwd(y, gy, ctx.act, None, ACT_NONE, g2)
+            gy = g2
+        c, np_, k = gy.shape[3], planes.shape[1], ctx.k
+        gw = ops.conv_planes_wide_wgrad(planes, gy, k, k // 2).view(c, np_, k, k)
+        gb = ops.colsum(gy).clone() if ctx.has_bias else None
+        return None, gw, gb, None
+
+
+class _WideToPlanes(torch.autograd.Function):
+    """nn.Conv2d(c, C, k, padding=k//2) (+ Tanh) -> fp32 planes ``[N, C, H, W]``, all C from one read of the input."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias, act):
+        np_, c, k = weight.shape[0], weight.shape[1], weight.shape[2]
+        wt = weight.detach().permute(0, 2, 3, 1).reshape(np_, k * k, c).contiguous()     # [C, taps, c]
+        y = ops.conv_wide_to_planes(x, wt, None if bias is None else bias.detach(), k, k // 2, act)
+        ctx.save_for_backward(x, weight, y)
+        ctx.k, ctx.act, ctx.has_bias = k, act, bias is not None
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        x, weight, y = ctx.saved_tensors
+        np_, c, k = weight.shape[0], weight.shape[1], ctx.k
+        g = gy.float().contiguous()
+        if ctx.act == ACT_TANH:
+            g = g * (1.0 - y * y)
+        gx = gw = gb = None
+        if ctx.needs_input_grad[0]:      # sum over the C gradient planes of the flipped convolution
+            wd = weight.detach().transpose(0, 1).reshape(c, np_ * k * k).contiguous()     # [c, C, taps]
+            gx = ops.conv_planes_to_wide(g, wd, None, k, k // 2, flip=True)
+        if ctx.needs_input_grad[1]:
+            dw = ops.conv_planes_wide_wgrad(g, x, k, k // 2, flip=True)                   # [c, C, taps]
+            gw = dw.transpose(0, 1).reshape(np_, c, k, k).contiguous()
+        if ctx.has_bias and ctx.needs_input_grad[2]:
+            gb = g.sum((0, 2, 3))
+        return gx, gw, gb, None
+
+
+class _Conv4x4s2InPlanes(torch.autograd.Function):
+    """nn.Conv2d(C, c, 4, 2, 1) on fp32 planes ``[N, C, H, W]``: tap-major im2col (16*C columns) + one pointwise GEMM."""
+
+    @staticmethod
+    def forward(ctx, planes, weight, bias):
+        from . import engine
+        n, np_, h, w = planes.shape
+        xcol = ops.im2col4x4_planes(planes, h // 2, w // 2, stride=2)
+        y = ops.pointwise_gemm(xcol, engine._thin_in_pack(weight), weight.shape[0],
+                               bias=None if bias is None else bias.detach(), k_valid=16 * np_)
+        ctx.save_for_backward(xcol)
+        ctx.np, ctx.has_bias = np_, bias is not None
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        (xcol,) = ctx.saved_tensors
+        gy = gy.contiguous()
+        c, np_ = gy.shape[-1], ctx.np
+        gw = ops.pointwise_wgrad(gy, xcol)[:, :16 * np_].reshape(c, 4, 4, np_).permute(0, 3, 1, 2).contiguous()
+        gb = ops.colsum(gy).clone() if ctx.has_bias else None
+        return None, gw, gb
+
+
+class _ConvT4x4s2OutPlanes(torch.autograd.Function):
+    """nn.ConvTranspose2d(c, C, 4, 2, 1) + Tanh -> fp32 planes ``[N, C, 2h, 2w]``: 16*C plane-major per-tap partial
+    products per input pixel (one GEMM over the wide input) + col2im with per-plane bias and Tanh."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias):
+        from . import engine
+        np_ = weight.shape[1]
+        part = ops.pointwise_gemm(x, engine._planes_out_fprop_pack(weight), 16 * np_, out_f32=True)
+        y = ops.col2im4x4s2_planes(part, np_, None if bias is None else bias.detach(), ACT_TANH)
+        ctx.save_for_backward(x, weight, y)
+        ctx.has_bias = bias is not None
+        return y
+
+    @staticmethod
+    def backward(ctx, g):
+        from . import engine
+        x, weight, y = ctx.saved_tensors
+        n, np_, h2, w2 = y.shape
+        g_pre = (g.float() * (1.0 - y * y)).contiguous()
+        cin = weight.shape[0]
+        gcol = ops.im2col4x4_planes(g_pre, h2 // 2, w2 // 2, stride=2)
+        gx = gw = gb = None
+        if ctx.needs_input_grad[0]:
+            gx = ops.pointwise_gemm(gcol, engine._planes_out_dgrad_pack(weight), cin, k_valid=16 * np_)
+        if ctx.needs_input_grad[1]:
+            gw = ops.pointwise_wgrad(x, gcol)[:, :16 * np_].reshape(cin, 4, 4, np_).permute(0, 3, 1, 2).contiguous()
+        if ctx.has_bias and ctx.needs_input_grad[2]:
+            gb = g_pre.sum((0, 2, 3))
+        return gx, gw, gb
+
+
 def conv4x4s2(x, mod: nn.Conv2d):
     if x.dim() == 3:
         if mod.in_channels != 1:
@@ -365,6 +497,19 @@ def convT4x4s2_out_tanh(x, mod: nn.ConvTranspose2d):
     if mod.out_channels != 1:
         raise RuntimeError("pai_b200: the B200 path produces 1-channel outputs; no fallback exists")
     return _ConvT4x4s2Out.apply(x, mod.weight, mod.bias)
+
+
+def conv4x4s2_in_planes(planes, mod: nn.Conv2d):
+    """First layer of the Attention U-Net on ``to_planes`` output ``[N, C, H, W]``, C = 1..4 (C = 1: use ``conv4x4s2``
+    on the ``to_plane`` plane)."""
+    _check_planes(mod.in_channels, "in_channels")
+    return _Conv4x4s2InPlanes.apply(planes, mod.weight, mod.bias)
+
+
+def convT4x4s2_out_planes_tanh(x, mod: nn.ConvTranspose2d):
+    """Last layer of the Attention U-Net -> fp32 ``[N, C, 2h, 2w]``, C = 1..4."""
+    _check_planes(mod.out_channels, "out_channels")
+    return _ConvT4x4s2OutPlanes.apply(x, mod.weight, mod.bias)
 
 
 class _ZeroGradFor(torch.autograd.Function):
@@ -431,6 +576,18 @@ def conv_out(x, mod: nn.Conv2d, act=ACT_NONE):
         raise RuntimeError("pai_b200: the B200 path produces 1-channel outputs; got "
                            f"out_channels={mod.out_channels}. No fallback exists.")
     return _WideToPlane.apply(x, mod.weight, mod.bias, act)
+
+
+def conv_in_planes(planes, mod: nn.Conv2d, act=ACT_NONE):
+    """``conv_in`` for ``to_planes`` output ``[N, C, H, W]``, C = 1..4."""
+    _check_planes(mod.in_channels, "in_channels")
+    return _PlanesToWide.apply(planes, mod.weight, mod.bias, act)
+
+
+def conv_out_planes(x, mod: nn.Conv2d, act=ACT_NONE):
+    """``conv_out`` -> fp32 ``[N, C, H, W]``, C = 1..4."""
+    _check_planes(mod.out_channels, "out_channels")
+    return _WideToPlanes.apply(x, mod.weight, mod.bias, act)
 
 
 # ------------------------------------------------------------------------------------------ BatchNorm (+activation)
@@ -885,3 +1042,13 @@ def to_plane(x: torch.Tensor) -> torch.Tensor:
     if x.dim() != 4 or x.shape[1] != 1:
         raise RuntimeError(f"pai_b200: expected a [N, 1, H, W] input, got {tuple(x.shape)}")
     return x.float().contiguous().view(x.shape[0], x.shape[2], x.shape[3])
+
+
+def to_planes(x: torch.Tensor, channels: int) -> torch.Tensor:
+    """``[N, C, H, W]`` network input with C == ``channels`` (1..4) -> contiguous fp32 planes ``[N, C, H, W]``."""
+    _check_planes(channels, "in_channels")
+    if not x.is_cuda:
+        raise RuntimeError("pai_b200: the B200 path needs CUDA tensors; there is no CPU fallback")
+    if x.dim() != 4 or x.shape[1] != channels:
+        raise RuntimeError(f"pai_b200: expected a [N, {channels}, H, W] input, got {tuple(x.shape)}")
+    return x.float().contiguous()

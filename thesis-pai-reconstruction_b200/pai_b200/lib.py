@@ -55,6 +55,8 @@ SIGNATURES = {
                            c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p],
     "pai_pointwise_wgrad": [c_void_p, c_ll, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p],
     "pai_col2im4x4s2": [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p],
+    "pai_im2col4x4_planes": [c_void_p, c_int, c_ll, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
+    "pai_col2im4x4s2_planes": [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_ll, c_void_p],
     "pai_conv3x3_fprop": [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_int, c_float,
                           c_void_p, c_int, c_int, c_int, c_void_p, c_void_p],
     "pai_conv3x3_wgrad": [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_void_p],
@@ -72,6 +74,12 @@ SIGNATURES = {
                                c_void_p, c_void_p],
     "pai_conv_plane_wide_wgrad": [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p,
                                   c_void_p],
+    "pai_conv_planes_to_wide": [c_void_p, c_int, c_ll, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
+                                c_int, c_int, c_float, c_void_p, c_int, c_void_p],
+    "pai_conv_wide_to_planes": [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int,
+                                c_void_p, c_int, c_ll, c_void_p],
+    "pai_conv_planes_wide_wgrad": [c_void_p, c_int, c_ll, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                                   c_int, c_void_p, c_void_p],
     "pai_gconv4_3x3_fprop": [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p],
     "pai_gconv4_3x3_wgrad": [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
     "pai_subsample2": [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p],

@@ -489,6 +489,37 @@ def im2col4x4(planes, oh, ow, stride=2, flip=False):
     return col
 
 
+def _planes(t: torch.Tensor):
+    """-> (n, np, h, w, plane_stride) of an fp32 NCHW stack of image planes ``[n, np, h, w]`` (plane j of image b at
+    element ``(b * np + j) * plane_stride``)."""
+    assert t.dim() == 4 and t.dtype == torch.float32, "expected fp32 planes [n, np, h, w]"
+    n, np_, h, w = t.shape
+    ps = t.stride(1) if np_ > 1 else (t.stride(0) if n > 1 else h * w)      # size-1 dimensions carry any stride
+    assert t.stride(3) == 1 and (h == 1 or t.stride(2) == w) and (n == 1 or t.stride(0) == np_ * ps) and ps >= h * w, \
+        f"not a plane stack: shape {tuple(t.shape)} strides {t.stride()}"
+    return n, np_, h, w, ps
+
+
+def im2col4x4_planes(planes, oh, ow, stride=2, flip=False):
+    """fp32 planes ``[n, np, ih, iw]`` (np <= 4) -> bf16 ``[n, oh, ow, 64]``, tap-major (channel = tap*np + j).  Only
+    the first ``16 * np`` channels are written (``k_valid=16 * np``)."""
+    n, np_, ih, iw, ps = _planes(planes)
+    col = torch.empty(n, oh, ow, 64, dtype=torch.bfloat16, device=planes.device)
+    lib.call("pai_im2col4x4_planes", _ptr(planes), np_, ps, n, ih, iw, oh, ow, stride, int(flip), _ptr(col), _stream())
+    return col
+
+
+def col2im4x4s2_planes(p, np_, bias=None, act=ACT_NONE):
+    """fp32 plane-major per-tap partial products ``[n, h, w, >=16*np]`` (column o*16 + tap) -> fp32 planes
+    ``[n, np, 2h, 2w]`` (transposed 4x4 stride-2 conv with np output channels)."""
+    n, h, w, c = p.shape
+    assert p.dtype == torch.float32 and p.stride(3) == 1 and c >= 16 * np_
+    out = torch.empty(n, np_, 2 * h, 2 * w, dtype=torch.float32, device=p.device)
+    lib.call("pai_col2im4x4s2_planes", _ptr(p), p.stride(2), n, h, w, _ptr(bias), act, _ptr(out), np_, 4 * h * w,
+             _stream())
+    return out
+
+
 def pointwise_gemm(x, w_packed, cout, bias=None, act=ACT_NONE, slope=0.2, out=None, out_f32=False, out2=None,
                    act2=ACT_NONE, n_tile=0, k_valid=0):
     """1x1 convolution: ``y[..., co] = act(bias + x[..., :] @ w_packed[co, :])`` over all pixels of an NHWC tensor.
@@ -725,6 +756,38 @@ def conv_plane_wide_wgrad(plane, wide, k, pad, flip=False):
     n, h, wd, c, ld = _nhwc(wide)
     dw = torch.zeros(c, k * k, dtype=torch.float32, device=wide.device)
     lib.call("pai_conv_plane_wide_wgrad", _ptr(plane), _ptr(wide), ld, n, h, wd, c, k, pad, int(flip), _ptr(dw), _stream())
+    return dw
+
+
+def conv_planes_to_wide(planes, w, bias, k, pad, act=ACT_NONE, slope=0.2, flip=False, out=None):
+    """planes fp32 ``[n, np, h, w]``, w fp32 ``[c, np*k*k]`` (Conv2d weight ``[c, np, k, k]``) -> NHWC bf16
+    ``[n, h, w, c]``; with ``flip`` the sum over the np planes is the data gradient of Conv2d(c, np, k)."""
+    n, np_, h, wd, ps = _planes(planes)
+    c = w.shape[0]
+    if out is None:
+        out = torch.empty(n, h, wd, c, dtype=torch.bfloat16, device=planes.device)
+    lib.call("pai_conv_planes_to_wide", _ptr(planes), np_, ps, n, h, wd, k, pad, int(flip), _ptr(w), _ptr(bias), c, act,
+             float(slope), _ptr(out), _nhwc(out)[4], _stream())
+    return out
+
+
+def conv_wide_to_planes(x, w, bias, k, pad, act=ACT_NONE):
+    """NHWC bf16 ``[n, h, w, c]``, w fp32 ``[np, k*k, c]`` -> fp32 planes ``[n, np, h, w]`` (one read of x)."""
+    n, h, wd, c, ld = _nhwc(x)
+    np_ = w.shape[0]
+    out = torch.empty(n, np_, h, wd, dtype=torch.float32, device=x.device)
+    lib.call("pai_conv_wide_to_planes", _ptr(x), n, h, wd, c, ld, k, pad, _ptr(w), _ptr(bias), act, _ptr(out), np_, h * wd,
+             _stream())
+    return out
+
+
+def conv_planes_wide_wgrad(planes, wide, k, pad, flip=False):
+    """-> fp32 ``[c, np, k*k]`` = sum over pixels of ``wide[p, c] * plane_j[p + off_t]``."""
+    _, np_, _, _, ps = _planes(planes)
+    n, h, wd, c, ld = _nhwc(wide)
+    dw = torch.zeros(c, np_, k * k, dtype=torch.float32, device=wide.device)
+    lib.call("pai_conv_planes_wide_wgrad", _ptr(planes), np_, ps, _ptr(wide), ld, n, h, wd, c, k, pad, int(flip), _ptr(dw),
+             _stream())
     return dw
 
 
