@@ -25,6 +25,8 @@ extern "C" {
 #define PAI_ACT_LEAKY 1 /* LeakyReLU(slope) */
 #define PAI_ACT_RELU 2
 #define PAI_ACT_TANH 3
+#define PAI_ACT_SIGMOID 4 /* fp32 check path only (pai_check_act_f32 / pai_check_act_bwd_f32) */
+#define PAI_ACT_GELU 5    /* exact erf GELU, fp32 check path only */
 
 #define PAI_DTYPE_F32 0
 #define PAI_DTYPE_BF16 1
@@ -470,6 +472,56 @@ int pai_check_conv2d_wgrad_f32(const float* x, int n, int cin, int h, int w, con
 int pai_check_batchnorm_bwd_f32(const float* x, const float* g, int n, int c, int hw, const float* gamma, float eps,
                                 float* dx, float* dgamma, float* dbeta, void* stream);
 int pai_check_act_bwd_f32(const float* x, const float* g, long long count, int act, float slope, float* dx, void* stream);
+/* The layers of the Residual / Attention / Trans U-Nets (fp32 NCHW or row-major [m, d] in and out, one thread per output;
+ * the convolution, Linear and attention sums add the exact fp32 products in double, in a fixed order; other reductions in
+ * double as above).  pai_check_act_f32 / pai_check_act_bwd_f32 also take
+ * PAI_ACT_SIGMOID (the attention gate) and PAI_ACT_GELU (the ViT feed-forward).
+ *   pai_check_conv2d_grouped_f32        pai_check_conv2d_f32 with groups (nn.Conv2d weight [cout,cin/groups,k,k],
+ *                                       nn.ConvTranspose2d weight [cin,cout/groups,k,k]) and, for transposed = 1, the
+ *                                       output_padding out_pad < stride.  The data gradient of a grouped Conv2d is the
+ *                                       grouped transposed convolution of g with the same weight (out_pad restores the
+ *                                       size a stride-2 forward rounded down).  groups = 1, out_pad = 0 computes
+ *                                       what pai_check_conv2d_f32 does, in the same order, with a double accumulator.
+ *   pai_check_conv2d_wgrad_grouped_f32  its weight gradient (layout of wt) and, if dbias != NULL, dbias[cout] = sum of g */
+int pai_check_conv2d_grouped_f32(const float* x, int n, int cin, int h, int w, const float* wt, int cout, int k,
+                                 int stride, int pad, int groups, int out_pad, const float* bias, int pre_act, float slope,
+                                 int transposed, float* y, void* stream);
+int pai_check_conv2d_wgrad_grouped_f32(const float* x, int n, int cin, int h, int w, const float* g, int cout, int k,
+                                       int stride, int pad, int groups, int out_pad, int pre_act, float slope, int transposed,
+                                       float* dw, float* dbias, void* stream);
+/*   pai_check_maxpool2_f32       nn.MaxPool2d(2) of x [n,c,h,w] -> y [n,c,h/2,w/2]
+ *   pai_check_maxpool2_bwd_f32   dx [n,c,h,w]: g goes to the first maximum of each 2x2 window in row-major order
+ *                                (torch's tie rule), every other element gets 0
+ *   pai_check_upsample2_f32      nn.Upsample(scale_factor=2) (nearest) of x [n,c,h,w] -> y [n,c,2h,2w]
+ *   pai_check_upsample2_bwd_f32  dx [n,c,h,w] = the sum of the 4 children of g [n,c,2h,2w], in row-major order */
+int pai_check_maxpool2_f32(const float* x, int n, int c, int h, int w, float* y, void* stream);
+int pai_check_maxpool2_bwd_f32(const float* x, const float* g, int n, int c, int h, int w, float* dx, void* stream);
+int pai_check_upsample2_f32(const float* x, int n, int c, int h, int w, float* y, void* stream);
+int pai_check_upsample2_bwd_f32(const float* g, int n, int c, int h, int w, float* dx, void* stream);
+/*   pai_check_layernorm_f32      nn.LayerNorm(d) over the rows of x [m,d]: mean and biased variance in double;
+ *                                also writes mean[m] and rstd[m] = 1/sqrt(var + eps) for the backward
+ *   pai_check_layernorm_bwd_f32  dx [m,d], dgamma [d], dbeta [d] from x, g and the forward's mean / rstd */
+int pai_check_layernorm_f32(const float* x, int m, int d, const float* gamma, const float* beta, float eps, float* y,
+                            float* mean, float* rstd, void* stream);
+int pai_check_layernorm_bwd_f32(const float* x, const float* g, int m, int d, const float* gamma, const float* mean,
+                                const float* rstd, float* dx, float* dgamma, float* dbeta, void* stream);
+/*   pai_check_linear_f32         nn.Linear with w [out,in]: transpose = 0: y [m,out] = x [m,in] w^T + bias;
+ *                                transpose = 1: y [m,in] = x [m,out] w (the data gradient; bias must be NULL)
+ *   pai_check_linear_wgrad_f32   dw [out,in] = g^T x, one thread per weight element reducing over the m rows;
+ *                                dbias [out] = column sums of g if dbias != NULL */
+int pai_check_linear_f32(const float* x, int m, int in, int out, const float* w, const float* bias, int transpose, float* y,
+                         void* stream);
+int pai_check_linear_wgrad_f32(const float* x, const float* g, int m, int in, int out, float* dw, float* dbias,
+                               void* stream);
+/*   pai_check_attention_f32      multi-head attention over the sequence axis of qkv [s*b, 3E] (row = i*b + batch index;
+ *                                Q | K | V column blocks, head h = columns [h*head_dim, (h+1)*head_dim), E = heads*head_dim,
+ *                                the layout of pai_attn_fwd): probs [b*heads, s, s] = softmax(Q K^T / sqrt(head_dim)) with
+ *                                max subtraction, out [s*b, E] = probs V
+ *   pai_check_attention_bwd_f32  dqkv [s*b, 3E] from qkv, the saved probs and dout [s*b, E]; ds_work [b*heads, s, s] */
+int pai_check_attention_f32(const float* qkv, int s, int b, int heads, int head_dim, float* probs, float* out,
+                            void* stream);
+int pai_check_attention_bwd_f32(const float* qkv, const float* probs, const float* dout, int s, int b, int heads,
+                                int head_dim, float* ds_work, float* dqkv, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * dataset.py's per-image transform (dataset.py:51-61,126-134) for a batch of decoded grayscale uint8 images [n,ih,iw]:

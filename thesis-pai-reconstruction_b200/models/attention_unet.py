@@ -13,7 +13,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from pai_b200 import layers as L, lib
+from pai_b200 import check, engine, layers as L, lib
 
 from .pix2pix import DecoderBlock, EncoderBlock
 from .wrapper import UnetWrapper
@@ -117,6 +117,8 @@ class AttentionUnet(nn.Module):
             return self._forward(x)
 
     def _forward(self, x):
+        if engine.check_path_enabled():                # exact fp32 kernels (pai_b200/check.py)
+            return check.attention_unet_forward(self, x)
         n, _, hh, ww = x.shape
         depth = len(self.encoders)
         if hh % (1 << depth) or ww % (1 << depth):

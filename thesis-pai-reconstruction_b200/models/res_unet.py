@@ -14,7 +14,7 @@ from typing import Literal, Sequence
 import torch
 import torch.nn as nn
 
-from pai_b200 import layers as L, lib
+from pai_b200 import check, engine, layers as L, lib
 
 from .wrapper import UnetWrapper
 
@@ -240,6 +240,8 @@ class ResUnet(nn.Module):
             return self._forward(x)
 
     def _forward(self, x):
+        if engine.check_path_enabled():                # exact fp32 kernels (pai_b200/check.py)
+            return check.res_unet_forward(self, x)
         n, _, hh, ww = x.shape
         depth = len(self.encoders)
         if hh % (1 << depth) or ww % (1 << depth):

@@ -21,7 +21,7 @@ import torch
 import torch.nn as nn
 from einops.layers.torch import Rearrange
 
-from pai_b200 import layers as L, lib
+from pai_b200 import check, engine, layers as L, lib
 
 from .wrapper import UnetWrapper
 
@@ -198,6 +198,8 @@ class TransUnet(nn.Module):
             return self._forward(x)
 
     def _forward(self, x):
+        if engine.check_path_enabled():                # exact fp32 kernels (pai_b200/check.py)
+            return check.trans_unet_forward(self, x)
         n, _, hh, ww = x.shape
         cin, cout = self.in_conv.in_channels, self.out[0].out_channels
         L.check_image_channels(cin, cout)

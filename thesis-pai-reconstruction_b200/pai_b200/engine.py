@@ -400,6 +400,117 @@ class _CheckAct(torch.autograd.Function):
         return ops.check_act_bwd(x, g.contiguous().float(), ctx.act, SLOPE), None
 
 
+class _CheckConv2d(torch.autograd.Function):
+    """``nn.Conv2d`` / ``nn.ConvTranspose2d`` with any stride, padding, groups and an optional bias (the Residual /
+    Attention / Trans U-Net layers) on ``pai_check_conv2d_grouped_f32``, which sums the exact fp32 products in double.
+    Data gradient of a Conv2d: the grouped transposed convolution of ``g`` with the same weight, with the output padding
+    that restores the rows / columns a strided forward rounded down; of a ConvTranspose2d: the convolution of ``g``."""
+
+    @staticmethod
+    def forward(ctx, x, w, b, stride, pad, groups, transposed):
+        y = ops.check_conv2d_grouped(x, w, b, stride=stride, pad=pad, groups=groups, transposed=transposed)
+        ctx.save_for_backward(x, w)
+        ctx.cfg = (stride, pad, groups, transposed, b is not None)
+        return y
+
+    @staticmethod
+    def backward(ctx, g):
+        x, w = ctx.saved_tensors
+        stride, pad, groups, transposed, has_b = ctx.cfg
+        g = g.contiguous().float()
+        gx = gw = gb = None
+        if ctx.needs_input_grad[0]:
+            out_pad = 0
+            if not transposed:
+                pads = [x.shape[d] - ((g.shape[d] - 1) * stride - 2 * pad + w.shape[2]) for d in (2, 3)]
+                if pads[0] != pads[1]:
+                    raise RuntimeError(f"pai_b200 check path: no data gradient for input {tuple(x.shape)} (stride {stride})")
+                out_pad = pads[0]
+            gx = ops.check_conv2d_grouped(g, w, None, stride=stride, pad=pad, groups=groups, out_pad=out_pad,
+                                          transposed=not transposed)
+            if gx.shape != x.shape:
+                raise RuntimeError(f"pai_b200 check path: data-gradient shape {tuple(gx.shape)} != input {tuple(x.shape)}")
+        if ctx.needs_input_grad[1] or (has_b and ctx.needs_input_grad[2]):
+            gw, gb = ops.check_conv2d_wgrad_grouped(x, g, tuple(w.shape), stride=stride, pad=pad, groups=groups,
+                                                    transposed=transposed, want_bias=has_b)
+        return gx, gw, gb, None, None, None, None
+
+
+class _CheckMaxPool2(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x):
+        ctx.save_for_backward(x)
+        return ops.check_maxpool2(x)
+
+    @staticmethod
+    def backward(ctx, g):
+        (x,) = ctx.saved_tensors
+        return ops.check_maxpool2_bwd(x, g.contiguous().float())
+
+
+class _CheckUpsample2(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x):
+        return ops.check_upsample2(x)
+
+    @staticmethod
+    def backward(ctx, g):
+        return ops.check_upsample2_bwd(g.contiguous().float())
+
+
+class _CheckLayerNorm(torch.autograd.Function):
+    """``nn.LayerNorm`` over the rows of ``x [m, d]``."""
+
+    @staticmethod
+    def forward(ctx, x, gamma, beta, eps):
+        y, mean, rstd = ops.check_layernorm(x, gamma.detach(), beta.detach(), eps)
+        ctx.save_for_backward(x, gamma, mean, rstd)
+        return y
+
+    @staticmethod
+    def backward(ctx, g):
+        x, gamma, mean, rstd = ctx.saved_tensors
+        dx, dgamma, dbeta = ops.check_layernorm_bwd(x, g.contiguous().float(), gamma.detach(), mean, rstd)
+        return dx, dgamma, dbeta, None
+
+
+class _CheckLinear(torch.autograd.Function):
+    """``nn.Linear``: ``x [m, in] -> x W^T + b``."""
+
+    @staticmethod
+    def forward(ctx, x, w, b):
+        ctx.save_for_backward(x, w)
+        ctx.has_b = b is not None
+        return ops.check_linear(x, w.detach(), None if b is None else b.detach())
+
+    @staticmethod
+    def backward(ctx, g):
+        x, w = ctx.saved_tensors
+        g = g.contiguous().float()
+        gx = gw = gb = None
+        if ctx.needs_input_grad[0]:
+            gx = ops.check_linear(g, w.detach(), transpose=True)
+        if ctx.needs_input_grad[1] or (ctx.has_b and ctx.needs_input_grad[2]):
+            gw, gb = ops.check_linear_wgrad(x, g, want_bias=ctx.has_b)
+        return gx, gw, gb
+
+
+class _CheckAttention(torch.autograd.Function):
+    """softmax(Q K^T / sqrt(hd)) V per head over the sequence axis of ``qkv [S*B, 3E]`` (the layout of ``L.attention``)."""
+
+    @staticmethod
+    def forward(ctx, qkv, s, b, heads):
+        out, probs = ops.check_attention(qkv, s, b, heads)
+        ctx.save_for_backward(qkv, probs)
+        ctx.dims = (s, b, heads)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        qkv, probs = ctx.saved_tensors
+        return ops.check_attention_bwd(qkv, probs, g.contiguous().float(), *ctx.dims), None, None, None
+
+
 def _check_bn(v, bn, training):
     if bn is None:
         return v

@@ -123,6 +123,21 @@ SIGNATURES = {
     "pai_check_batchnorm_bwd_f32": [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_float, c_void_p, c_void_p, c_void_p,
                                     c_void_p],
     "pai_check_act_bwd_f32": [c_void_p, c_void_p, c_ll, c_int, c_float, c_void_p, c_void_p],
+    "pai_check_conv2d_grouped_f32": [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int,
+                                     c_int, c_void_p, c_int, c_float, c_int, c_void_p, c_void_p],
+    "pai_check_conv2d_wgrad_grouped_f32": [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int,
+                                           c_int, c_int, c_int, c_float, c_int, c_void_p, c_void_p, c_void_p],
+    "pai_check_maxpool2_f32": [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
+    "pai_check_maxpool2_bwd_f32": [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
+    "pai_check_upsample2_f32": [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
+    "pai_check_upsample2_bwd_f32": [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p],
+    "pai_check_layernorm_f32": [c_void_p, c_int, c_int, c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_void_p, c_void_p],
+    "pai_check_layernorm_bwd_f32": [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                    c_void_p, c_void_p],
+    "pai_check_linear_f32": [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p],
+    "pai_check_linear_wgrad_f32": [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p],
+    "pai_check_attention_f32": [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p],
+    "pai_check_attention_bwd_f32": [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p],
     "pai_thin_conv4x4s2_fprop": [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p, c_int,
                                  c_int, c_void_p, c_int, c_int, c_float, c_void_p],
     "pai_thin_conv4x4s2_wgrad": [c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p],

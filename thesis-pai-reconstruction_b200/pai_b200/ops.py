@@ -14,6 +14,7 @@ import torch
 from . import lib
 
 ACT_NONE, ACT_LEAKY, ACT_RELU, ACT_TANH = 0, 1, 2, 3
+ACT_SIGMOID, ACT_GELU = 4, 5           # fp32 check path only (check_act / check_act_bwd)
 BN_SMALL_OFF = os.environ.get("PAI_NO_BN_SMALL", "0") == "1"
 # ConvTranspose2d(4,2,1) sub-pixel phases (SURVEY.md Appendix B): T[parity] = ((k, d), (k, d))
 _T_K = ((1, 3), (0, 2))
@@ -999,3 +1000,136 @@ def check_act_bwd(x, g, act, slope=0.2):
     dx = torch.empty_like(x)
     lib.call("pai_check_act_bwd_f32", _ptr(x), _ptr(g), x.numel(), act, slope, _ptr(dx), _stream())
     return dx
+
+
+def check_conv2d_grouped(x, w, bias=None, stride=1, pad=1, groups=1, out_pad=0, pre_act=ACT_NONE, slope=0.2,
+                         transposed=False):
+    """``check_conv2d`` with ``groups`` (weight [cout, cin/groups, k, k], transposed: [cin, cout/groups, k, k]) and a
+    transposed convolution's ``output_padding``."""
+    assert x.dtype == torch.float32 and w.dtype == torch.float32 and x.is_cuda
+    x, w = x.contiguous(), w.contiguous()
+    n, cin, h, wd = x.shape
+    k = w.shape[2]
+    cout = w.shape[1] * groups if transposed else w.shape[0]
+    assert w.shape[2] == w.shape[3] and (w.shape[0] if transposed else w.shape[1] * groups) == cin
+    ho = (h - 1) * stride - 2 * pad + k + out_pad if transposed else (h + 2 * pad - k) // stride + 1
+    wo = (wd - 1) * stride - 2 * pad + k + out_pad if transposed else (wd + 2 * pad - k) // stride + 1
+    y = torch.empty(n, cout, ho, wo, dtype=torch.float32, device=x.device)
+    b = None if bias is None else bias.contiguous()
+    lib.call("pai_check_conv2d_grouped_f32", _ptr(x), n, cin, h, wd, _ptr(w), cout, k, stride, pad, groups, out_pad, _ptr(b),
+             pre_act, slope, 1 if transposed else 0, _ptr(y), _stream())
+    return y
+
+
+def check_conv2d_wgrad_grouped(x, g, w_shape, stride=1, pad=1, groups=1, out_pad=0, pre_act=ACT_NONE, slope=0.2,
+                               transposed=False, want_bias=True):
+    """-> (dW in the weight's own layout, dbias or None) of ``y = conv(pre_act(x), groups)`` given ``g = dL/dy``."""
+    x, g = x.contiguous(), g.contiguous()
+    n, cin, h, wd = x.shape
+    cout, k = g.shape[1], w_shape[2]
+    dw = torch.empty(w_shape, dtype=torch.float32, device=x.device)
+    db = torch.empty(cout, dtype=torch.float32, device=x.device) if want_bias else None
+    lib.call("pai_check_conv2d_wgrad_grouped_f32", _ptr(x), n, cin, h, wd, _ptr(g), cout, k, stride, pad, groups, out_pad,
+             pre_act, slope, 1 if transposed else 0, _ptr(dw), _ptr(db), _stream(), kernels=2 if want_bias else 1)
+    return dw, db
+
+
+def check_maxpool2(x):
+    x = x.contiguous()
+    n, c, h, w = x.shape
+    y = torch.empty(n, c, h // 2, w // 2, dtype=torch.float32, device=x.device)
+    lib.call("pai_check_maxpool2_f32", _ptr(x), n, c, h, w, _ptr(y), _stream())
+    return y
+
+
+def check_maxpool2_bwd(x, g):
+    x, g = x.contiguous(), g.contiguous()
+    n, c, h, w = x.shape
+    dx = torch.empty_like(x)
+    lib.call("pai_check_maxpool2_bwd_f32", _ptr(x), _ptr(g), n, c, h, w, _ptr(dx), _stream())
+    return dx
+
+
+def check_upsample2(x):
+    x = x.contiguous()
+    n, c, h, w = x.shape
+    y = torch.empty(n, c, 2 * h, 2 * w, dtype=torch.float32, device=x.device)
+    lib.call("pai_check_upsample2_f32", _ptr(x), n, c, h, w, _ptr(y), _stream())
+    return y
+
+
+def check_upsample2_bwd(g):
+    g = g.contiguous()
+    n, c, h2, w2 = g.shape
+    dx = torch.empty(n, c, h2 // 2, w2 // 2, dtype=torch.float32, device=g.device)
+    lib.call("pai_check_upsample2_bwd_f32", _ptr(g), n, c, h2 // 2, w2 // 2, _ptr(dx), _stream())
+    return dx
+
+
+def check_layernorm(x, gamma, beta, eps=1e-5):
+    """-> (y, mean, rstd) of LayerNorm over the rows of fp32 ``x [m, d]``."""
+    x = x.contiguous()
+    m, d = x.shape
+    y = torch.empty_like(x)
+    mean = torch.empty(m, dtype=torch.float32, device=x.device)
+    rstd = torch.empty(m, dtype=torch.float32, device=x.device)
+    lib.call("pai_check_layernorm_f32", _ptr(x), m, d, _ptr(gamma.contiguous()), _ptr(beta.contiguous()), float(eps), _ptr(y),
+             _ptr(mean), _ptr(rstd), _stream())
+    return y, mean, rstd
+
+
+def check_layernorm_bwd(x, g, gamma, mean, rstd):
+    x, g = x.contiguous(), g.contiguous()
+    m, d = x.shape
+    dx = torch.empty_like(x)
+    dgamma = torch.empty(d, dtype=torch.float32, device=x.device)
+    dbeta = torch.empty(d, dtype=torch.float32, device=x.device)
+    lib.call("pai_check_layernorm_bwd_f32", _ptr(x), _ptr(g), m, d, _ptr(gamma.contiguous()), _ptr(mean), _ptr(rstd), _ptr(dx),
+             _ptr(dgamma), _ptr(dbeta), _stream(), kernels=2)
+    return dx, dgamma, dbeta
+
+
+def check_linear(x, w, bias=None, transpose=False):
+    """``x W^T + b`` (x [m, in]) or, with ``transpose``, ``x W`` (x [m, out]: the data gradient) for W [out, in]."""
+    x, w = x.contiguous(), w.contiguous()
+    out, inn = w.shape
+    m = x.shape[0]
+    assert x.shape[1] == (out if transpose else inn)
+    y = torch.empty(m, inn if transpose else out, dtype=torch.float32, device=x.device)
+    lib.call("pai_check_linear_f32", _ptr(x), m, inn, out, _ptr(w), _ptr(None if bias is None else bias.contiguous()),
+             1 if transpose else 0, _ptr(y), _stream())
+    return y
+
+
+def check_linear_wgrad(x, g, want_bias=True):
+    """-> (dW [out, in], dbias [out] or None) of ``y = x W^T + b`` given ``g = dL/dy``."""
+    x, g = x.contiguous(), g.contiguous()
+    m, inn = x.shape
+    out = g.shape[1]
+    dw = torch.empty(out, inn, dtype=torch.float32, device=x.device)
+    db = torch.empty(out, dtype=torch.float32, device=x.device) if want_bias else None
+    lib.call("pai_check_linear_wgrad_f32", _ptr(x), _ptr(g), m, inn, out, _ptr(dw), _ptr(db), _stream())
+    return dw, db
+
+
+def check_attention(qkv, s, b, heads):
+    """-> (out [s*b, E], probs [b*heads, s, s]) of multi-head attention over the sequence axis of fp32 ``qkv [s*b, 3E]``."""
+    qkv = qkv.contiguous()
+    e = qkv.shape[1] // 3
+    assert qkv.dim() == 2 and qkv.shape == (s * b, 3 * e) and e % heads == 0, (tuple(qkv.shape), s, b, heads)
+    probs = torch.empty(b * heads, s, s, dtype=torch.float32, device=qkv.device)
+    out = torch.empty(s * b, e, dtype=torch.float32, device=qkv.device)
+    lib.call("pai_check_attention_f32", _ptr(qkv), s, b, heads, e // heads, _ptr(probs), _ptr(out), _stream(), kernels=2)
+    return out, probs
+
+
+def check_attention_bwd(qkv, probs, dout, s, b, heads):
+    qkv, dout = qkv.contiguous(), dout.contiguous()
+    e = qkv.shape[1] // 3
+    assert qkv.dim() == 2 and qkv.shape == (s * b, 3 * e) and e % heads == 0, (tuple(qkv.shape), s, b, heads)
+    assert dout.shape == (s * b, e) and probs.shape == (b * heads, s, s), (tuple(dout.shape), tuple(probs.shape))
+    ds = torch.empty_like(probs)
+    dqkv = torch.empty_like(qkv)
+    lib.call("pai_check_attention_bwd_f32", _ptr(qkv), _ptr(probs), _ptr(dout), s, b, heads, e // heads, _ptr(ds), _ptr(dqkv),
+             _stream(), kernels=2)
+    return dqkv
